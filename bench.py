@@ -1,8 +1,14 @@
 #!/usr/bin/env python
 """bench.py -- headline benchmark of the B200 cproc renderer.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl native|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl native|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
+
+--dump-outputs DIR writes what the last timed step computed (rank 0's shard) to
+DIR/<name>.npy, so that two builds can be compared output for output.  On the
+native path the inputs depend only on the arguments.  The reference arm sizes
+its sample by the host's core count, so its dumps compare only between runs on
+hosts with the same number of cores.
 
 Workload (BASELINE.json configs[1], SURVEY.md section 8d "C2"): the PDM
 sigma-delta modulator, 65,536 independent channels x 16 Mi samples, integer,
@@ -41,6 +47,9 @@ E2E_TICKS = 1024 * 1024              # e2e step: 65,536 ch x 1 Mi samples throug
 # device-to-host stream of a rank drops from 57 to 46 GB/s as soon as a second rank streams too, and to 11 GB/s per rank
 # at eight (measured; plain concurrent copies into 1 GiB buffers do not show it) -- the DMA working set, not the fabric.
 E2E_CHUNK = int(os.environ.get("E2E_CHUNK_TICKS", "4096"))
+DUMP_CHANNELS = 256                  # --dump-outputs: seeded sample of channels whose duty is written tick by tick
+DUMP_TICKS = 8192                    # ... over the last ticks of each launch written
+DUMP_MAX_BYTES = 64 << 20
 
 
 def measured_peaks():
@@ -146,6 +155,10 @@ def run_reference(args, rank, world):
     for _ in range(args.steps):
         _, count = lib.pdm_v2_run(chan, 2, n_ch, 3, prng, None, 0x3FF, count, CTL_LOG, 24, sp, ticks, out=duty)
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        idx = dump_channels(n_ch)
+        write_outputs(args.dump_outputs, {"duty_channels": idx, "duty": duty[idx, -DUMP_TICKS:], "duty_sum": duty.sum(axis=1),
+                                          "channel_state": chan, "bank_prng": prng, "bank_count": np.array([count], np.uint32)})
     value = n_ch * ticks * args.steps / dt
     sample = "%d ch x %d samples per step (same modulator, setpoints and dither as the native arm), gcc -O2, output buffer preallocated" % (n_ch, ticks)
     line = {
@@ -165,6 +178,51 @@ def workload_config():
                         "4096 ticks): 65,536 channels x 16 Mi samples per GPU, uint8 duty out",
             "channels_per_gpu": N_CH, "samples_per_channel": F_TOTAL, "launch_ticks": F_CHUNK,
             "out_layout": "TILED [t/16][ch][16]", "l2": "inputs+outputs larger than L2 (8 GiB output slab per launch)"}
+
+
+# --------------------------------------------------------------------------- --dump-outputs
+def dump_channels(n_ch):
+    """The channels whose duty --dump-outputs writes tick by tick: a fixed, seeded, sorted sample."""
+    import numpy as np
+    return np.sort(np.random.default_rng(20261020).choice(n_ch, size=min(DUMP_CHANNELS, n_ch), replace=False))
+
+
+def write_outputs(path, arrays):
+    """DIR/<name>.npy per array: 8- and 16-bit integers as float32, wider integers as float64 (both exact)."""
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    out = {}
+    for name, a in arrays.items():
+        a = np.asarray(a)
+        out[name] = a.astype(np.float32 if a.dtype.kind == "f" or a.dtype.itemsize <= 2 else np.float64)
+    total = sum(a.nbytes for a in out.values())
+    assert total <= DUMP_MAX_BYTES, "dump of %d bytes exceeds %d" % (total, DUMP_MAX_BYTES)
+    for name, a in out.items():
+        np.save(os.path.join(path, name + ".npy"), a)
+    print("bench: wrote %d arrays (%.1f MB) to %s" % (len(out), total / 1e6, path), file=sys.stderr)
+
+
+def dump_native(path, torch, batch, slabs, n_chunks):
+    """What the last timed step leaves its caller: the duty of its last two launches (the two slabs alternate, so these are
+    the two still in HBM) -- tick by tick for the sampled channels over each launch's last DUMP_TICKS ticks, and summed
+    over all ticks for every channel -- and the channel and dither-bank state the step ends with."""
+    import numpy as np
+    idx = dump_channels(N_CH)
+    sel = torch.from_numpy(idx).to(slabs[0].device)
+    arrays = {"duty_channels": idx}
+    for name, k in (("prev_launch", n_chunks - 2), ("last_launch", n_chunks - 1)):
+        tiles = slabs[k & 1].view(F_CHUNK // 16, N_CH, 16)                      # TILED: [t/16][ch][16]
+        win = tiles[-(DUMP_TICKS // 16):].index_select(1, sel)
+        arrays[name + "_duty"] = win.permute(1, 0, 2).reshape(len(idx), DUMP_TICKS).cpu().numpy()
+        total = torch.zeros(N_CH, dtype=torch.int64, device=slabs[0].device)
+        for r in range(0, F_CHUNK // 16, 512):                                  # int32 partial sums of 512 x 16 bytes
+            total += tiles[r:r + 512].sum(dim=(0, 2), dtype=torch.int32)
+        arrays[name + "_duty_sum"] = total.cpu().numpy()
+    prng, count = batch.download_bank()
+    arrays["channel_state"] = batch.download_state()
+    arrays["bank_prng"] = prng
+    arrays["bank_count"] = np.array([count], np.uint32)
+    write_outputs(path, arrays)
 
 
 # --------------------------------------------------------------------------- native arm
@@ -295,6 +353,8 @@ def run_native(args, rank, local_rank, world):
     ms_max = float(t.item())
     ms_per_step = ms_max / args.steps
     value = world * N_CH * F_TOTAL / (ms_per_step * 1e-3)
+    if args.dump_outputs and rank == 0:
+        dump_native(args.dump_outputs, torch, batch, slabs, n_chunks)    # before the e2e leg runs the batch on
 
     # ---- end to end through the C-ABI with HOST buffers: setpoints H2D, duty D2H
     e2e_rows = E2E_TICKS >> CTL_LOG
@@ -423,7 +483,11 @@ def main():
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="native", choices=["native", "reference"])
     ap.add_argument("--no-other-configs", action="store_true", help="skip the secondary configuration rows (N=1)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one computed to DIR/<name>.npy (float32/float64, <= 64 MB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     # stdout carries the ONE JSON line and nothing else: libraries that write to fd 1 (NCCL prints its version
     # banner there) are sent to stderr, the line goes to the saved descriptor.  The re-exec below inherits fd 1.
     global _JSON_OUT
@@ -440,6 +504,8 @@ def main():
         cmd = [sys.executable, "-m", "torch.distributed.run", "--nnodes=1", "--nproc-per-node", str(args.gpus),
                "--master-addr", "127.0.0.1", "--master-port", port, os.path.abspath(__file__),
                "--gpus", str(args.gpus), "--steps", str(args.steps), "--warmup", str(args.warmup)]
+        cmd += ["--no-other-configs"] if args.no_other_configs else []
+        cmd += ["--dump-outputs", args.dump_outputs] if args.dump_outputs else []
         sys.exit(subprocess.call(cmd))
     sys.stdout.flush()
     _JSON_OUT = os.fdopen(os.dup(1), "w")

@@ -164,6 +164,12 @@ class _Lib:
           ctl_div_log, out_shift, _ptr(setpoints), F, _ptr(duty))
         return duty, cnt.value
 
+    def pwm_run(self, phase, speed, N, F):
+        duty = np.zeros((N, F), np.uint8)
+        f = self._fn("pwm_run", None, [VP, VP, C.c_uint64, C.c_uint64, VP])
+        f(_ptr(phase), _ptr(speed), N, F, _ptr(duty))
+        return duty
+
     def square_grain_run(self, state, threshold, N, F, inp, out=None):
         if out is None:
             out = np.zeros((N, F), np.float32)
@@ -202,12 +208,6 @@ class Oracle(_Lib):
         f.argtypes = [VP, C.c_uint32, C.c_uint32, C.POINTER(C.c_uint32), C.c_uint32, C.c_uint64, VP]
         f(_ptr(chan), chan.shape[0], pin_chan0, C.byref(r), dmask, F, _ptr(gpio))
         return gpio, r.value
-
-    def pwm_run(self, phase, speed, N, F):
-        duty = np.zeros((N, F), np.uint8)
-        f = self._fn("pwm_run", None, [VP, VP, C.c_uint64, C.c_uint64, VP])
-        f(_ptr(phase), _ptr(speed), N, F, _ptr(duty))
-        return duty
 
     def note_to_inc(self, note):
         return self._fn("note_to_inc", C.c_uint32, [C.c_int])(note)

@@ -7,7 +7,6 @@ bit for bit, the graph TEXT compiled as C equals the parsed node table run by th
 fused extension voice (orc_xvoice_tick).  GPU: the CUDA graph path equals the oracle bit for bit in every layout and
 kernel variant, and the voice graph equals k_xvoice's raw output."""
 import os
-import shutil
 
 import numpy as np
 import pytest
@@ -113,18 +112,12 @@ def test_ext_oracle_restatement_equals_the_def_proc_bodies(ref, oracle, seed):
     assert np.array_equal(a, b) and np.array_equal(sa, sb), rows
 
 
-def _private_ref(tmp_path):
-    priv = str(tmp_path / "libref_private.so")                     # node state is function-static: one instance per loaded copy
-    shutil.copy(po.REF_SO, priv)
-    return po.Ref(priv)
-
-
-def test_graph_text_compiled_as_c_equals_the_parsed_table(ref, oracle, tmp_path):
+def test_graph_text_compiled_as_c_equals_the_parsed_table(ref, oracle):
     """tests/golden/ext_voice.cproc and ext_chain.cproc: the SAME text compiled with the reference's PROC / PROC_COND
     macros (oracle/ref/ref_ext_voice.c) and parsed by cproc_cuda_graph_parse + run by the oracle."""
     rng = np.random.default_rng(5)
     F = 700
-    r = _private_ref(tmp_path)
+    r = ref.private_copy()                                       # node state is function-static: one instance per loaded copy
     # voice: input[0] = pitch modulation
     g = abi.graph_parse_ex(VOICE_TEXT)
     assert g["out_is_float"] == [True, True] and g["out_indices"] == [0, 1] and g["n_inputs"] == 1

@@ -19,11 +19,7 @@ def test_struct_sizes(ref):
 def test_test_cproc_anchor(ref, oracle):
     """linux/test_cproc.c graph: inputs 0,1,1,0,0,1,0,1,1,1,0 -> n2.out = 0,1,1,2,2,3,4,5,5,5,6.
     The reference keeps its state in function statics, so load a private copy."""
-    import shutil, tempfile, os
-    d = tempfile.mkdtemp()
-    p = os.path.join(d, "libref_private.so")
-    shutil.copy(po.REF_SO, p)
-    r = po.Ref(p)
+    r = ref.private_copy()
     seq = [0, 1, 1, 0, 0, 1, 0, 1, 1, 1, 0]
     got = [r.test_cproc_tick(x, 1) for x in seq]
     assert [g[0] for g in got] == [2] * len(seq)          # cproc_output(2, ...)
@@ -140,9 +136,7 @@ def test_pwm_update_oracle_vs_ref(ref, oracle):
     sp[0] = 256 * 13                                         # the firmware's default speed (:160)
     pa, pb = ph.copy(), ph.copy()
     a = oracle.pwm_run(pa, sp.copy(), N, F)
-    b = np.zeros((N, F), np.uint8)
-    f = ref._fn("pwm_run", None, [po.VP, po.VP, po.C.c_uint64, po.C.c_uint64, po.VP])
-    f(po._ptr(pb), po._ptr(sp), N, F, po._ptr(b))
+    b = ref.pwm_run(pb, sp.copy(), N, F)
     assert np.array_equal(a, b) and np.array_equal(pa, pb)
 
 
