@@ -651,9 +651,10 @@ __global__ void k_xvoice_final(const float *partial, float *mix, uint64_t n_bloc
 //          maps, sequential over the C chunks of a variant because C is small.
 // Pass 3 (k_sweep_render) then runs the ordinary bit-exact float tick from each start
 // state.  The start states come from exact arithmetic rather than from the float
-// trajectory, so raw output matches the sequential path to rounding noise of the
-// float recurrence, not bit for bit: tolerance <= 1e-5 of peak, >= 120 dB SNR
-// (tests/test_gpu_parity.py::test_xvoice_scan).  phase, t and env stay bit-exact.
+// trajectory, so the raw output is not bit for bit the sequential path's: per voice it is
+// within 1e-5 of the voice's own peak of the fp64 filter, or within twice the sequential
+// render's own error where that is larger (measured on a B200: <= 1.3e-6, slow and
+// resonant filters included; tests/test_gpu_float_ref.py).  phase, t and env stay bit-exact.
 struct SweepParams {
     XVoiceParams x;
     uint64_t L, C;
@@ -1229,8 +1230,12 @@ struct OnepoleOp {
 //   pass 1  zero-state response z_c of each full chunk, fp64, same recurrence       (k_onepole_zsr)
 //   pass 2  y_{c+1} = (1 - a)^L y_c + z_c, fp64, sequential over the C chunks        (k_onepole_scan)
 //   pass 3  the ordinary float tick from each chunk's start state                    (k_onepole_render)
-// Start states come from exact arithmetic rather than the float trajectory: outputs match the
-// sequential kernel to <= 1e-5 of peak / >= 120 dB SNR (tests: test_onepole_scan), not bit for bit.
+// Start states come from exact arithmetic rather than the float trajectory, so outputs are not bit
+// for bit the sequential kernel's: every instance is within 1e-5 of its own peak of the fp64
+// recurrence, or within twice the sequential render's error where that is larger (measured on a
+// B200: <= 4.7e-6 for 2^-24 <= a <= 1.999; tests/test_gpu_float_ref.py).  The sequential float
+// tick stalls where |a (x - y)| < 1/2 ulp(y) (small coefficients) and drifts up to 1.8e-3 of the
+// peak from the exact result there; the scan only drifts within one chunk.
 struct OnepoleScanParams {
     float *y; const float *a;
     uint64_t n, F, L, C;

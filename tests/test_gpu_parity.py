@@ -1030,8 +1030,10 @@ def test_xvoice_mix_only(st, ctx, oracle, N, F, mixgen):
 @pytest.mark.parametrize("layout,groups", [("TILED", 4), ("PLANAR", 1), ("PLANAR", 3)])
 def test_xvoice_scan_zero_state_forms(st, ctx, oracle, closed, layout, groups):
     """The closed-form zero-state pass (per phase wrap) and the ticked fp64 pass give chunk start states
-    inside the same tolerance, for every kind of increment: none, one wrap per 2^32 ticks, powers of two,
-    increments past 2^31 (a wrap nearly every tick), gaps of exactly k and of k+1 ticks."""
+    inside the same tolerance of the sequential oracle (1e-5 of the peak, benign filters), for every kind of
+    increment: none, one wrap per 2^32 ticks, powers of two, increments past 2^31 (a wrap nearly every tick),
+    gaps of exactly k and of k+1 ticks.  The same set at the slow filter f = 1e-3, voice by voice against the
+    fp64 filter: tests/test_gpu_float_ref.py::test_xvoice_scan_slow_filter_increments."""
     special = np.array([0, 1, 2, 3, 1 << 20, 1 << 24, (1 << 24) + 1, (1 << 24) - 1, 3 << 28, 1 << 31, (1 << 31) + 5, (1 << 31) - 1,
                         0xFFFFFFFF, 0xFFFFFFFE, 0x12345678, 0x9ABCDEF0, 0x55555555, 0x55555556, 0x00F00F00, 715827883], np.uint32)
     N, F = 512, 1536
@@ -1063,7 +1065,8 @@ def test_xvoice_scan_zero_state_forms(st, ctx, oracle, closed, layout, groups):
 @pytest.mark.parametrize("N,F,chunk,groups,mode", [(70, 1001, 32, 0, 2), (200, 3000, 96, 0, 1), (700, 2048, 32, 3, 1), (40, 2050, 64, 0, 2), (500, 998, 32, 4, 2)])
 def test_xvoice_scan_planar_store_paths(st, ctx, oracle, N, F, chunk, groups, mode):
     """PLANAR render: tensor-TMA stores (planar_bulk 2, even F) and the staged-row kernel it falls back to
-    (odd F, planar_bulk 1) agree with the sequential oracle to the stated tolerance."""
+    (odd F, planar_bulk 1) agree with the sequential oracle to 1e-5 of the peak at benign filters (the
+    per-voice contract against the fp64 filter: tests/test_gpu_float_ref.py)."""
     s0, prm = _xvoice_inputs(oracle, N)
     prm["gate_frames"] = rng.integers(0, F, N)
     sa = s0.copy()
@@ -1090,8 +1093,11 @@ def test_xvoice_scan_planar_store_paths(st, ctx, oracle, N, F, chunk, groups, mo
                                               (700, 2048, 64, 0), (700, 2048, 32, 3), (300, 1024, 512, 1), (129, 640, 64, 8), (1100, 1056, 96, 0), (1100, 1056, 96, 5)])
 def test_xvoice_scan(st, ctx, oracle, layout, N, F, chunk, groups):
     """Time-parallel raw render: chunk start states from the fp64 scan of the SVF's affine
-    recurrence.  phase / t / env bit-exact; lp, bp and the output within <= 1e-5 of the
-    peak and >= 120 dB SNR of the sequential oracle (stated tolerance of BASELINE.json)."""
+    recurrence.  phase / t / env bit-exact; at these benign filters (f 0.01..0.3, q 0.5..2), where the
+    sequential render is itself within ~1e-6 of the exact filter, lp, bp and the output stay within
+    <= 1e-5 of the peak and >= 120 dB SNR of the sequential oracle, for every chunking and grouping.
+    The accuracy contract itself -- per voice against the fp64 filter, slow and resonant filters
+    included -- is tests/test_gpu_float_ref.py."""
     s0, prm = _xvoice_inputs(oracle, N)
     prm["gate_frames"] = rng.integers(0, F, N)
     prm["env_release"] = rng.uniform(2e-4, 1e-2, N)
@@ -1152,8 +1158,12 @@ def test_onepole(st, ctx, oracle, layout, N, F):
 @pytest.mark.parametrize("layout", ["PLANAR", "INTERLEAVED"])
 @pytest.mark.parametrize("N,F,chunk", [(1, 100000, 0), (3, 65536, 0), (40, 5000, 96), (130, 777, 50), (2, 64, 0)])
 def test_onepole_scan(st, ctx, oracle, layout, N, F, chunk):
-    """Time-parallel one-pole (block scan of the affine recurrence over the time axis): within the
-    stated tolerance of the sequential oracle, final state included."""
+    """Time-parallel one-pole (block scan of the affine recurrence over the time axis): at these
+    coefficients (a 5e-4..0.5 on noise plus a slow sine), where the sequential render does not stall and
+    is itself within ~1e-6 of the exact recurrence, within 1e-5 of the peak / 120 dB SNR of the
+    sequential oracle, final state included.  At small coefficients the sequential float render drifts
+    from the exact result and the scan is the more accurate of the two: the contract against the fp64
+    recurrence, instance by instance, is tests/test_gpu_float_ref.py."""
     inp = rng.uniform(-1, 1, (N, F)).astype(np.float32)
     inp += np.sin(np.arange(F) * 0.001).astype(np.float32)            # slow component: the filter output is not just noise
     a = rng.uniform(0.0005, 0.5, (N, 1)).astype(np.float32)
