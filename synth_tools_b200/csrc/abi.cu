@@ -120,8 +120,6 @@ int cproc_cuda_set_option(cproc_cuda_ctx *ctx, const char *name, int64_t value) 
     else if (!strcmp(name, "planar_bulk")) { if (value < 0 || value > 2) return cproc_set_err(ctx, CPROC_CUDA_EINVAL, "planar_bulk must be 0..2"); ctx->planar_bulk = (int)value; }
     else if (!strcmp(name, "graph_vec4")) ctx->graph_vec4 = value != 0;
     else if (!strcmp(name, "graph_jit")) ctx->graph_jit = value != 0;
-    else if (!strcmp(name, "grain_bulk")) { if (value < 0 || value > 5) return cproc_set_err(ctx, CPROC_CUDA_EINVAL, "grain_bulk must be 0..5"); ctx->grain_bulk = (int)value; }
-    else if (!strcmp(name, "grain_vec4")) ctx->grain_vec4 = value != 0;
     else if (!strcmp(name, "grain_mix2")) { if (value < 0 || value > 2) return cproc_set_err(ctx, CPROC_CUDA_EINVAL, "grain_mix2 must be 0..2"); ctx->grain_mix2 = (int)value; }
     else if (!strcmp(name, "xvoice_chunk")) { if (value < 0) return cproc_set_err(ctx, CPROC_CUDA_EINVAL, "xvoice_chunk must be >= 0"); ctx->xvoice_chunk = (int)value; }
     else if (!strcmp(name, "xvoice_vpt")) { if (value < 0 || value > 65536) return cproc_set_err(ctx, CPROC_CUDA_EINVAL, "xvoice_vpt must be 0..65536"); ctx->xvoice_vpt = (int)value; }
@@ -426,7 +424,6 @@ int cproc_cuda_run(cproc_cuda_batch *b, uint64_t F, const cproc_cuda_io *io) {
     const bool zc_ok = io->layout == CPROC_CUDA_PLANAR && ctx->planar_bulk >= 1 &&
         (proc == CPROC_CUDA_VOICE_BANK ? io->mix == nullptr
          : proc == CPROC_CUDA_PWM ? F % 16 == 0
-         : proc == CPROC_CUDA_SQUARE_GRAIN ? (F % 4 == 0 && ctx->grain_bulk != 0)
          : F % 4 == 0);
     // run_graph 3: no graph and no copies -- direct launches on the pinned staging (one launch + one sync per period)
     if (ctx->run_graph >= 3 && graphable && zc_ok && sz.in + sz.in2 + sz.ctl + sz.out + sz.mix <= (64u << 10)) {

@@ -38,10 +38,8 @@ struct cproc_cuda_ctx {
     int voice_fpt = 0;        // voice bank: frames per thread (0 = by frame count; 1, 2, 4, 8)
     int grain_block = 128;
     int grain_blocks_per_sm = 2;
-    int grain_bulk = 5;       // planar square_grain: 0 register-transpose kernel; 1..4 per-lane bulk-copy kernel (tile/stage shapes); 5 tensor-TMA kernel
-    int grain_vec4 = 1;       // interleaved square_grain: four grains per thread when n % 4 == 0
     int grain_mix2 = 2;       // 0: float kernel; 1: register-accumulator / integer-threshold kernel; 2: predicate-state kernel
-    int planar_bulk = 2;      // PLANAR pdm_raw / onepole / pwm streams through planar_bulk.cuh: 0 off, 1 per-lane bulk copies, 2 tensor TMA
+    int planar_bulk = 2;      // square_grain / pdm_raw / onepole / pwm streams through planar_bulk.cuh: 0 off, 1 per-lane bulk copies, 2 tensor TMA (PLANAR); nonzero: k_interleaved4 (INTERLEAVED)
     int graph_vec4 = 1;       // interleaved generated graphs: four instances per thread when n % 4 == 0
     int graph_jit = 1;        // 1: generated graphs are compiled with NVRTC; 0: table-driven kernel
     int xvoice_vpt = 0;       // k_xvoice_mix: voices per thread per L2-resident tile (0 = default)

@@ -15,7 +15,7 @@
 //    generates CUDA source for exactly this graph (every node state word a named
 //    register, every source a literal register name, masks as immediates) and compiles
 //    it with NVRTC for sm_100a when the batch is created.  PLANAR streams are staged
-//    with per-lane bulk copies as in k_grain_bulk; INTERLEAVED streams are read in
+//    with per-lane bulk copies as in pbulk::k_planar_bulk; INTERLEAVED streams are read in
 //    16-frame batches.  libnvrtc is loaded with dlopen: without it (or with graph_jit=0)
 //    graphs of up to 16 nodes run on the table-driven kernel of k_graph.cu.
 #include "common.cuh"
@@ -433,7 +433,7 @@ extern "C" __global__ void __launch_bounds__(128) graph_interleaved(const GraphP
 }
 
 // Four adjacent instances per thread (128-bit accesses): a block covers 2 KiB of every stream row
-// instead of 512 B -- fewer distant row segments and pages per block (see k_grain_interleaved4).
+// instead of 512 B -- fewer distant row segments and pages per block (see pbulk::k_interleaved4).
 // n % 4 == 0, 16-byte aligned streams.
 #define GI4_B 4
 extern "C" __global__ void __launch_bounds__(128) graph_interleaved4(const GraphParams p) {

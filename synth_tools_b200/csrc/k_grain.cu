@@ -9,15 +9,18 @@
 // hysteresis makes the recurrence a 3-state machine that is serial in time;
 // the grain axis carries the parallelism (one thread per grain).
 //
-// k_grain_planar: hosts hand over planar [grain][F] vectors.  A warp owns 32
-//   grains and walks the frame axis in 32-frame tiles: the tile is loaded with
-//   32 coalesced 128-byte row reads into padded shared memory, each lane then
-//   runs its own grain along its row IN PLACE (in may alias out, as in Pd),
-//   and the tile is written back with 32 coalesced row stores.
-// k_grain_interleaved: [F][grain] streams are already coalesced.
+// GrainOp: PLANAR [grain][F] streams go through the staging templates of
+//   planar_bulk.cuh (k_planar_tma, k_planar_bulk), INTERLEAVED [F][grain] streams
+//   through k_interleaved4 (four grains per thread), as the other stream processors.
+// k_grain_planar: the PLANAR fallback (planar_bulk = 0, F % 4 != 0 or rows off
+//   16-byte alignment).  A warp owns 32 grains and walks the frame axis in 32-frame
+//   tiles: the tile is loaded with 32 coalesced 128-byte row reads into padded
+//   shared memory, each lane then runs its own grain along its row IN PLACE (in may
+//   alias out, as in Pd), and the tile is written back with 32 coalesced row stores.
+// k_grain_interleaved: the INTERLEAVED fallback, one grain per thread.
 // k_grain_mix: config C3b -- input from a per-grain phasor, integer stereo mix.
 #include "common.cuh"
-#include <cuda.h>
+#include "planar_bulk.cuh"
 
 struct GrainParams {
     float *state;            // SoA [1][npad]
@@ -33,6 +36,16 @@ __device__ __forceinline__ float grain_step(float &state, float val, float thres
     else if (state < 0.0f && val > thresh) state = 0.5f;     // :95-97
     return o;
 }
+
+// one grain as an Op of the PLANAR / INTERLEAVED stream templates (planar_bulk.cuh)
+struct GrainOp {
+    static constexpr int NIN = 1;
+    float *state; const float *thresh;
+    float st, th;
+    __device__ __forceinline__ void load(uint64_t i) { st = state[i]; th = thresh[i]; }
+    __device__ __forceinline__ void store(uint64_t i) { state[i] = st; }
+    __device__ __forceinline__ uint32_t tick(uint32_t x, uint64_t) { return __float_as_uint(grain_step(st, __uint_as_float(x), th)); }
+};
 
 #define GRAIN_WARPS 4
 __global__ void __launch_bounds__(GRAIN_WARPS * 32) k_grain_planar(const GrainParams p) {
@@ -63,8 +76,7 @@ __global__ void __launch_bounds__(GRAIN_WARPS * 32) k_grain_planar(const GrainPa
 // [F][grain] streams: a warp's 32 grains are 128 contiguous bytes of every frame row.
 // in and out may be the same buffer, so the compiler cannot move loads across stores:
 // the 16-frame batches make the independent loads explicit (all in flight, then the
-// serial trigger steps, then the stores).  Dynamic shared memory is requested only to
-// pin the number of resident blocks per SM (see grain_residency).
+// serial trigger steps, then the stores).
 #define GI_BLOCK 128
 #define GI_BATCH 16
 __global__ void __launch_bounds__(GI_BLOCK) k_grain_interleaved(const GrainParams p) {
@@ -91,339 +103,29 @@ __global__ void __launch_bounds__(GI_BLOCK) k_grain_interleaved(const GrainParam
     p.state[g] = state;
 }
 
-// Four adjacent grains per thread (128-bit loads/stores): a block covers 2 KiB of every
-// frame row, which quarters the number of distant row segments (and pages) a block walks.
-#ifndef GI4_BATCH
-#define GI4_BATCH 8
-#endif
-#ifndef GI4_MINB
-#define GI4_MINB 1
-#endif
-__global__ void __launch_bounds__(GI_BLOCK, GI4_MINB) k_grain_interleaved4(const GrainParams p) {
-    const uint64_t g = ((uint64_t)blockIdx.x * blockDim.x + threadIdx.x) * 4;
-    if (g >= p.n) return;                                    // n % 4 == 0
-    float4 st = *(const float4 *)(p.state + g);
-    const float4 th = *(const float4 *)(p.thresh + g);
-    const float *src = p.in + g;
-    float *dst = p.out + g;
-    auto step4 = [&](float4 v) {
-        float4 o;
-        o.x = grain_step(st.x, v.x, th.x); o.y = grain_step(st.y, v.y, th.y);
-        o.z = grain_step(st.z, v.z, th.z); o.w = grain_step(st.w, v.w, th.w);
-        return o;
-    };
-    uint64_t t = 0;
-    for (; t + GI4_BATCH <= p.F; t += GI4_BATCH) {
-        float4 v[GI4_BATCH];
-#pragma unroll
-        for (int i = 0; i < GI4_BATCH; ++i) v[i] = __ldcs((const float4 *)(src + (t + i) * p.n));
-#pragma unroll
-        for (int i = 0; i < GI4_BATCH; ++i) v[i] = step4(v[i]);
-#pragma unroll
-        for (int i = 0; i < GI4_BATCH; ++i) __stcs((float4 *)(dst + (t + i) * p.n), v[i]);
-    }
-    for (; t < p.F; ++t) __stcs((float4 *)(dst + t * p.n), step4(__ldcs((const float4 *)(src + t * p.n))));
-    *(float4 *)(p.state + g) = st;
-}
-
-// Blocks of equal duration run in rounds of (SMs x resident blocks): pick the residency
-// (within [r_min, r_max]) whose last round is fullest, and the shared-memory request that
-// makes the hardware hold exactly that many blocks per SM.
-static int grain_residency(uint64_t blocks, int n_sm, int r_min, int r_max, size_t *smem) {
-    int best = r_max; double best_eff = 0.0;
-    for (int r = r_max; r >= r_min; --r) {
-        const uint64_t per_round = (uint64_t)n_sm * r;
-        const double eff = (double)blocks / (double)(per_round * ceil_div_u64(blocks, per_round));
-        if (eff > best_eff + 0.01) { best_eff = eff; best = r; }
-    }
-    *smem = (size_t)(227 * 1024) / best - 1024;          // 1 KiB per block is reserved by the system
-    return best;
-}
-
-// ---------------------------------------------------------------------------
-// k_grain_bulk: the planar layout without a register transpose.  Lane r of a warp
-// owns grain r of the warp's 32.  Per tile of TF frames every lane issues ONE bulk
-// copy (cp.async.bulk, the non-tensor TMA path) of its own row segment -- TF*4
-// contiguous bytes of HBM -- into its row of a shared-memory stage; a per-stage
-// mbarrier counts the bytes in.  The lane then walks its row with LDS.128 /
-// STS.128 (row stride TF*4+16 bytes: the 16-byte units of 8 consecutive lanes fall
-// in 8 different bank groups) and sends the row back with one bulk store.  Loads
-// run one tile ahead of the compute, stores drain one tile behind it.  No thread
-// touches another thread's data, so the only synchronisation is the mbarrier.
-// `in` may alias `out` exactly (Pd in-place): a row segment is always read before
-// it is written.
-__device__ __forceinline__ uint32_t smem_u32(const void *p) { return (uint32_t)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void mbar_init(uint32_t bar, uint32_t count) { asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(bar), "r"(count)); }
-__device__ __forceinline__ void mbar_expect_tx(uint32_t bar, uint32_t bytes) {
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity) {
-    asm volatile("{\n\t.reg .pred p;\n\t"
-                 "W: mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n\t"
-                 "@p bra D;\n\tbra W;\n\tD:\n\t}" ::"r"(bar), "r"(parity) : "memory");
-}
-__device__ __forceinline__ void bulk_g2s(uint32_t dst, const void *src, uint32_t bytes, uint32_t bar) {
-    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-                 ::"r"(dst), "l"(src), "r"(bytes), "r"(bar) : "memory");
-}
-__device__ __forceinline__ void bulk_s2g(void *dst, uint32_t src, uint32_t bytes) {
-    asm volatile("cp.async.bulk.global.shared::cta.bulk_group [%0], [%1], %2;" ::"l"(dst), "r"(src), "r"(bytes) : "memory");
-}
-
-// One frame of the fast form: state is the predicate `neg`; valid for state = +-0.5 and
-// thresh >= 0 (then at most one of the two flip conditions holds, synth_tools.c:92-97).
-__device__ __forceinline__ float grain_step_p(bool &neg, float val, float th, float nth) {
-    const float o = neg ? -0.5f : 0.5f;                      // :91
-    neg = (val < nth) | (neg & !(val > th));
-    return o;
-}
-
-#define GB_WARPS 2
-template <int TF, int STAGES>
-__global__ void __launch_bounds__(GB_WARPS * 32) k_grain_bulk(const GrainParams p) {
-    constexpr uint32_t ROWB = TF * 4 + 16;
-    constexpr uint32_t STAGEB = 32 * ROWB;
-    extern __shared__ __align__(128) uint8_t gb_smem[];
-    const uint32_t lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    const uint64_t g0 = ((uint64_t)blockIdx.x * GB_WARPS + warp) * 32;
-    if (g0 >= p.n) return;
-    const uint32_t rows = p.n - g0 < 32 ? (uint32_t)(p.n - g0) : 32u;
-    const bool mine = lane < rows;
-    const uint32_t base = smem_u32(gb_smem) + warp * (STAGES * STAGEB);
-    const uint32_t bar0 = smem_u32(gb_smem) + GB_WARPS * STAGES * STAGEB + warp * (STAGES * 8);
-    if (lane == 0) {
-#pragma unroll
-        for (int s = 0; s < STAGES; ++s) mbar_init(bar0 + 8 * s, 1);
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
-    __syncwarp();
-    float state = mine ? p.state[g0 + lane] : 0.5f;
-    const float th = mine ? p.thresh[g0 + lane] : 0.0f;
-    const float nth = -th;
-    const float *src = p.in + (g0 + lane) * p.F;
-    float *dst = p.out + (g0 + lane) * p.F;
-    const uint32_t n_tiles = (uint32_t)((p.F + TF - 1) / TF);
-    auto cols_of = [&](uint32_t k) { const uint64_t left = p.F - (uint64_t)k * TF; return left < TF ? (uint32_t)left : (uint32_t)TF; };
-    auto issue = [&](uint32_t k) {
-        const uint32_t s = k % STAGES, bytes = cols_of(k) * 4;
-        if (lane == 0) mbar_expect_tx(bar0 + 8 * s, rows * bytes);
-        if (mine) bulk_g2s(base + s * STAGEB + lane * ROWB, src + (uint64_t)k * TF, bytes, bar0 + 8 * s);
-    };
-#pragma unroll 1
-    for (uint32_t k = 0; k < STAGES - 2 && k < n_tiles; ++k) issue(k);
-#pragma unroll 1
-    for (uint32_t k = 0; k < n_tiles; ++k) {
-        // the stage tile k+STAGES-2 lands in last held tile k-2: its bulk store must have read it out
-        if (k + STAGES - 2 < n_tiles) {
-            asm volatile("cp.async.bulk.wait_group.read 1;" ::: "memory");
-            __syncwarp();
-            issue(k + STAGES - 2);
-        }
-        const uint32_t s = k % STAGES, cols = cols_of(k);
-        mbar_wait(bar0 + 8 * s, (k / STAGES) & 1);
-        const uint32_t row = base + s * STAGEB + lane * ROWB;
-        if (mine) {
-            if ((state == 0.5f || state == -0.5f) && th >= 0.0f && cols == TF) {
-                bool neg = state < 0.0f;
-#pragma unroll 4
-                for (uint32_t c = 0; c < TF / 4; ++c) {
-                    float4 v;
-                    asm volatile("ld.shared.v4.f32 {%0, %1, %2, %3}, [%4];" : "=f"(v.x), "=f"(v.y), "=f"(v.z), "=f"(v.w) : "r"(row + 16 * c));
-                    v.x = grain_step_p(neg, v.x, th, nth); v.y = grain_step_p(neg, v.y, th, nth);
-                    v.z = grain_step_p(neg, v.z, th, nth); v.w = grain_step_p(neg, v.w, th, nth);
-                    asm volatile("st.shared.v4.f32 [%0], {%1, %2, %3, %4};" ::"r"(row + 16 * c), "f"(v.x), "f"(v.y), "f"(v.z), "f"(v.w) : "memory");
-                }
-                state = neg ? -0.5f : 0.5f;
-            } else {
-                // initial 0.0 (or any other) state value, negative threshold, ragged last tile: literal form
-                for (uint32_t c = 0; c < cols / 4; ++c) {
-                    float4 v;
-                    asm volatile("ld.shared.v4.f32 {%0, %1, %2, %3}, [%4];" : "=f"(v.x), "=f"(v.y), "=f"(v.z), "=f"(v.w) : "r"(row + 16 * c));
-                    v.x = grain_step(state, v.x, th); v.y = grain_step(state, v.y, th);
-                    v.z = grain_step(state, v.z, th); v.w = grain_step(state, v.w, th);
-                    asm volatile("st.shared.v4.f32 [%0], {%1, %2, %3, %4};" ::"r"(row + 16 * c), "f"(v.x), "f"(v.y), "f"(v.z), "f"(v.w) : "memory");
-                }
-            }
-            asm volatile("fence.proxy.async.shared::cta;" ::: "memory");     // generic-proxy row writes -> visible to the bulk store
-            bulk_s2g(dst + (uint64_t)k * TF, row, cols * 4);
-        }
-        asm volatile("cp.async.bulk.commit_group;" ::: "memory");
-    }
-    asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");
-    if (mine) p.state[g0 + lane] = state;
-}
-
-template <int TF, int STAGES>
-static int launch_grain_bulk(cproc_cuda_ctx *ctx, const GrainParams &p) {
-    constexpr size_t smem = (size_t)GB_WARPS * STAGES * 32 * (TF * 4 + 16) + GB_WARPS * STAGES * 8;
-    static bool attr_set[64] = {};
-    if (!attr_set[ctx->device & 63]) {
-        CK(ctx, cudaFuncSetAttribute(k_grain_bulk<TF, STAGES>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        attr_set[ctx->device & 63] = true;
-    }
-    k_grain_bulk<TF, STAGES><<<(unsigned)ceil_div_u64(p.n, GB_WARPS * 32), GB_WARPS * 32, smem, ctx->stream>>>(p);
-    return 0;
-}
-
-// ---------------------------------------------------------------------------
-// k_grain_tma: the same lane-owns-a-row scheme with TENSOR TMA.  k_grain_bulk issues one bulk copy
-// per lane, which the hardware's uniform datapath executes one lane at a time (the SASS loops over
-// the 32 lanes around every UBLKCP: ~640 of the ~900 warp instructions per tile are copy issue).
-// Here the [grain][frame] stream is described once per launch by a 2-D tensor map (box = 32 frames
-// x 32 grains = one 128-byte row segment per lane, SWIZZLE_128B) and ONE elected lane issues two
-// cp.async.bulk.tensor loads and two stores per 64-frame tile.  The 128-byte swizzle XORs the
-// 16-byte chunk index with (row & 7): lane r finds chunk c of its row at r*128 + ((c ^ (r & 7)) << 4),
-// so the LDS.128 / STS.128 of eight consecutive lanes fall in eight different bank groups.
-// Out-of-range rows / frames are zero-filled on load and clipped on store by the TMA unit.
-#define GT_WARPS 2
-#define GT_STAGES 3
-#define GT_BOXB 4096                       // 32 rows x 128 B
-#define GT_STAGEB (2 * GT_BOXB)            // 64 frames
-__global__ void __launch_bounds__(GT_WARPS * 32) k_grain_tma(const GrainParams p, const __grid_constant__ CUtensorMap tm_in, const __grid_constant__ CUtensorMap tm_out) {
-    extern __shared__ __align__(1024) uint8_t gt_smem[];
-    const uint32_t lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    const uint64_t g0 = ((uint64_t)blockIdx.x * GT_WARPS + warp) * 32;
-    if (g0 >= p.n) return;
-    const uint32_t rows = p.n - g0 < 32 ? (uint32_t)(p.n - g0) : 32u;
-    const bool mine = lane < rows;
-    const uint32_t sm0 = (smem_u32(gt_smem) + 1023u) & ~1023u;                 // swizzle atoms are 1 KiB
-    const uint32_t base = sm0 + warp * (GT_STAGES * GT_STAGEB);
-    const uint32_t bar0 = sm0 + GT_WARPS * GT_STAGES * GT_STAGEB + warp * (GT_STAGES * 8);
-    if (lane == 0) {
-#pragma unroll
-        for (int s = 0; s < GT_STAGES; ++s) mbar_init(bar0 + 8 * s, 1);
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
-    __syncwarp();
-    float state = mine ? p.state[g0 + lane] : 0.5f;
-    const float th = mine ? p.thresh[g0 + lane] : 0.0f;
-    const float nth = -th;
-    const uint32_t n_tiles = (uint32_t)((p.F + 63) / 64);
-    const uint64_t tmi = reinterpret_cast<uint64_t>(&tm_in), tmo = reinterpret_cast<uint64_t>(&tm_out);
-    auto cols_of = [&](uint32_t k) { const uint64_t left = p.F - (uint64_t)k * 64; return left < 64 ? (uint32_t)left : 64u; };
-    auto issue = [&](uint32_t k) {                                             // lane 0 only
-        const uint32_t s = k % GT_STAGES, nbox = cols_of(k) > 32 ? 2u : 1u;
-        mbar_expect_tx(bar0 + 8 * s, nbox * GT_BOXB);
-        for (uint32_t h = 0; h < nbox; ++h)
-            asm volatile("cp.async.bulk.tensor.2d.shared::cluster.global.tile.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3}], [%4];"
-                         ::"r"(base + s * GT_STAGEB + h * GT_BOXB), "l"(tmi), "r"((int32_t)(k * 64 + h * 32)), "r"((int32_t)g0), "r"(bar0 + 8 * s) : "memory");
-    };
-    if (lane == 0) for (uint32_t k = 0; k < GT_STAGES - 2 && k < n_tiles; ++k) issue(k);
-#pragma unroll 1
-    for (uint32_t k = 0; k < n_tiles; ++k) {
-        if (k + GT_STAGES - 2 < n_tiles) {                                     // that stage last held tile k-2: its stores must have read it out
-            if (lane == 0) { asm volatile("cp.async.bulk.wait_group.read 1;" ::: "memory"); issue(k + GT_STAGES - 2); }
-        }
-        const uint32_t s = k % GT_STAGES, cols = cols_of(k);
-        mbar_wait(bar0 + 8 * s, (k / GT_STAGES) & 1);
-        if (mine) {
-            const bool fast = (state == 0.5f || state == -0.5f) && th >= 0.0f;
-            bool neg = state < 0.0f;
-            for (uint32_t c = 0; c < cols / 4; ++c) {
-                const uint32_t a = base + s * GT_STAGEB + (c >> 3) * GT_BOXB + lane * 128 + (((c & 7) ^ (lane & 7)) << 4);
-                float4 v;
-                asm volatile("ld.shared.v4.f32 {%0, %1, %2, %3}, [%4];" : "=f"(v.x), "=f"(v.y), "=f"(v.z), "=f"(v.w) : "r"(a));
-                if (fast) {
-                    v.x = grain_step_p(neg, v.x, th, nth); v.y = grain_step_p(neg, v.y, th, nth);
-                    v.z = grain_step_p(neg, v.z, th, nth); v.w = grain_step_p(neg, v.w, th, nth);
-                } else {                                                       // initial 0.0 (or any other) state value, negative threshold: literal form
-                    v.x = grain_step(state, v.x, th); v.y = grain_step(state, v.y, th);
-                    v.z = grain_step(state, v.z, th); v.w = grain_step(state, v.w, th);
-                }
-                asm volatile("st.shared.v4.f32 [%0], {%1, %2, %3, %4};" ::"r"(a), "f"(v.x), "f"(v.y), "f"(v.z), "f"(v.w) : "memory");
-            }
-            if (fast) state = neg ? -0.5f : 0.5f;
-        }
-        asm volatile("fence.proxy.async.shared::cta;" ::: "memory");          // generic-proxy writes -> visible to the TMA store
-        __syncwarp();
-        if (lane == 0) {
-            const uint32_t nbox = cols > 32 ? 2u : 1u;
-            for (uint32_t h = 0; h < nbox; ++h)
-                asm volatile("cp.async.bulk.tensor.2d.global.shared::cta.tile.bulk_group [%0, {%1, %2}], [%3];"
-                             ::"l"(tmo), "r"((int32_t)(k * 64 + h * 32)), "r"((int32_t)g0), "r"(base + s * GT_STAGEB + h * GT_BOXB) : "memory");
-            asm volatile("cp.async.bulk.commit_group;" ::: "memory");
-        }
-    }
-    if (lane == 0) asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");
-    __syncwarp();
-    if (mine) p.state[g0 + lane] = state;
-}
-
-typedef CUresult (*cuTensorMapEncodeTiled_t)(CUtensorMap *, CUtensorMapDataType, cuuint32_t, void *, const cuuint64_t *, const cuuint64_t *, const cuuint32_t *,
-                                             const cuuint32_t *, CUtensorMapInterleave, CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-static cuTensorMapEncodeTiled_t grain_encode_fn() {
-    static cuTensorMapEncodeTiled_t fn = nullptr;
-    static bool tried = false;
-    if (!tried) {
-        tried = true;
-        void *q = nullptr;
-        cudaDriverEntryPointQueryResult qr;
-        if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &q, cudaEnableDefault, &qr) == cudaSuccess && qr == cudaDriverEntryPointSuccess) fn = (cuTensorMapEncodeTiled_t)q;
-        else cudaGetLastError();
-    }
-    return fn;
-}
-
-// returns 1 when the TMA kernel was launched, 0 when the caller should use another kernel, < 0 on error
-static int launch_grain_tma(cproc_cuda_ctx *ctx, const GrainParams &p) {
-    cuTensorMapEncodeTiled_t enc = grain_encode_fn();
-    if (!enc) return 0;
-    CUtensorMap tin, tout;
-    const cuuint64_t dims[2] = {p.F, p.n}, strides[1] = {p.F * sizeof(float)};
-    const cuuint32_t box[2] = {32, 32}, estr[2] = {1, 1};
-    if (enc(&tin, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 2, (void *)p.in, dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B,
-            CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) != CUDA_SUCCESS) return 0;
-    if (enc(&tout, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 2, (void *)p.out, dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B,
-            CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) != CUDA_SUCCESS) return 0;
-    constexpr size_t smem = (size_t)GT_WARPS * GT_STAGES * GT_STAGEB + GT_WARPS * GT_STAGES * 8 + 1024;
-    static bool attr_set[64] = {};
-    if (!attr_set[ctx->device & 63]) {
-        CK(ctx, cudaFuncSetAttribute(k_grain_tma, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        attr_set[ctx->device & 63] = true;
-    }
-    k_grain_tma<<<(unsigned)ceil_div_u64(p.n, GT_WARPS * 32), GT_WARPS * 32, smem, ctx->stream>>>(p, tin, tout);
-    return 1;
-}
-
 int launch_square_grain(cproc_cuda_batch *b, uint64_t F, const cproc_cuda_io *io) {
     cproc_cuda_ctx *ctx = b->ctx;
     if (!io->in || !io->out) return cproc_set_err(ctx, CPROC_CUDA_EINVAL, "square_grain: in/out is NULL");
     if (io->layout == CPROC_CUDA_TILED) return cproc_set_err(ctx, CPROC_CUDA_EINVAL, "square_grain: TILED layout not supported");
     if (F == 0) return 0;
+    GrainOp op; op.state = (float *)b->d_state; op.thresh = (const float *)b->d_param; op.st = 0.f; op.th = 0.f;
+    if (ctx->planar_bulk && io->layout == CPROC_CUDA_PLANAR && pbulk::usable(F, io->in, io->out)) {
+        int rc = pbulk::launch<64, 3>(ctx, op, (const uint32_t *)io->in, (uint32_t *)io->out, b->n, F);
+        if (rc) return rc;
+        CK_LAUNCH(ctx, "k_grain (bulk)");
+        return 0;
+    }
+    if (ctx->planar_bulk && io->layout == CPROC_CUDA_INTERLEAVED && pbulk::usable_interleaved4(b->n, io->in, io->out)) {
+        pbulk::launch_interleaved4(ctx, op, (const uint32_t *)io->in, (uint32_t *)io->out, b->n, F);
+        CK_LAUNCH(ctx, "k_grain (interleaved4)");
+        return 0;
+    }
     GrainParams p;
     p.state = (float *)b->d_state; p.thresh = (const float *)b->d_param; p.n = b->n; p.F = F;
     p.in = (const float *)io->in; p.out = (float *)io->out;
-    // bulk copies move 16-byte units: rows must start and end on 16-byte boundaries
-    const bool bulk_ok = ctx->grain_bulk && F % 4 == 0 && ((uintptr_t)p.in & 15) == 0 && ((uintptr_t)p.out & 15) == 0;
-    if (io->layout == CPROC_CUDA_INTERLEAVED) {
-        const bool vec4 = ctx->grain_vec4 && p.n % 4 == 0 && ((uintptr_t)p.in & 15) == 0 && ((uintptr_t)p.out & 15) == 0;
-        const uint64_t blocks = ceil_div_u64(p.n, vec4 ? GI_BLOCK * 4 : GI_BLOCK);
-        size_t smem = 0;
-        grain_residency(blocks, ctx->n_sm, 6, 16, &smem);
-        static bool attr_set[64] = {};
-        if (!attr_set[ctx->device & 63]) {
-            CK(ctx, cudaFuncSetAttribute(k_grain_interleaved, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024 / 6));
-            CK(ctx, cudaFuncSetAttribute(k_grain_interleaved4, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024 / 6));
-            attr_set[ctx->device & 63] = true;
-        }
-        if (vec4) k_grain_interleaved4<<<(unsigned)blocks, GI_BLOCK, smem, ctx->stream>>>(p);
-        else k_grain_interleaved<<<(unsigned)blocks, GI_BLOCK, smem, ctx->stream>>>(p);
-    } else if (bulk_ok) {
-        int rc = 0;
-        // tensor TMA: rows of F * 4 bytes must be 16-byte multiples (F % 4, checked) and fewer than 2^32 elements per dimension
-        if (ctx->grain_bulk == 5 && p.F < (1ull << 31) && p.n < (1ull << 31)) {
-            rc = launch_grain_tma(ctx, p);
-            if (rc < 0) return rc;
-        }
-        if (rc == 1) { /* launched */ }
-        else switch (ctx->grain_bulk) {
-        case 2: rc = launch_grain_bulk<128, 3>(ctx, p); break;
-        case 3: rc = launch_grain_bulk<64, 4>(ctx, p); break;
-        case 4: rc = launch_grain_bulk<32, 4>(ctx, p); break;
-        default: rc = launch_grain_bulk<64, 3>(ctx, p); break;
-        }
-        if (rc < 0) return rc;
-    } else
+    if (io->layout == CPROC_CUDA_INTERLEAVED)
+        k_grain_interleaved<<<(unsigned)ceil_div_u64(p.n, GI_BLOCK), GI_BLOCK, 0, ctx->stream>>>(p);
+    else
         k_grain_planar<<<(unsigned)ceil_div_u64(p.n, GRAIN_WARPS * 32), GRAIN_WARPS * 32, 0, ctx->stream>>>(p);
     CK_LAUNCH(ctx, "k_grain");
     return 0;

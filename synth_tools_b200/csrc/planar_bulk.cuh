@@ -1,6 +1,6 @@
 // planar_bulk.cuh -- generic bulk-staged render of PLANAR 32-bit streams ([inst][F], what
-// the reference hosts hand over).  The scheme of k_grain_bulk (k_grain.cu) as a template:
-// lane r of a warp owns instance r of the warp's 32; per tile of TF frames the lane issues
+// the reference hosts hand over), shared by square_grain, pdm raw, pwm, the one-pole and the
+// word clock.  Lane r of a warp owns instance r of the warp's 32; per tile of TF frames the lane issues
 // one bulk copy (cp.async.bulk, the non-tensor TMA path) of ITS row segment into its row
 // of a shared-memory stage, walks the row with LDS.128 / STS.128 in place, and sends it
 // back with one bulk store.  Loads run one tile ahead, stores drain one tile behind.

@@ -881,28 +881,29 @@ def test_square_grain(st, ctx, oracle, N, F, layout):
     _square_grain_case(st, ctx, oracle, N, F, layout)
 
 
-@pytest.mark.parametrize("vec4", [0, 1])
+@pytest.mark.parametrize("mode", [0, 2], ids=["planar_bulk=0", "planar_bulk=2"])
 @pytest.mark.parametrize("N,F", [(1000, 256), (64, 7), (4100, 40), (1001, 33)])
-def test_square_grain_interleaved_variants(st, ctx, oracle, vec4, N, F):
-    ctx.set_option("grain_vec4", vec4)
+def test_square_grain_interleaved_variants(st, ctx, oracle, mode, N, F):
+    """k_interleaved4<GrainOp> (planar_bulk 2, n % 4 == 0) and the one-grain-per-thread kernel."""
+    ctx.set_option("planar_bulk", mode)
     try:
         _square_grain_case(st, ctx, oracle, N, F, "INTERLEAVED", True, True)
     finally:
-        ctx.set_option("grain_vec4", 1)
+        ctx.set_option("planar_bulk", 2)
 
 
-@pytest.mark.parametrize("bulk", [0, 1, 2, 3, 4, 5])
+@pytest.mark.parametrize("mode", [0, 1, 2])
 @pytest.mark.parametrize("N,F,neg_th,odd", [(1000, 256, False, False), (77, 100, False, False), (300, 1024, True, False),
                                             (64, 4, False, True), (4097, 64, True, True), (31, 392, False, False)])
-def test_square_grain_bulk_variants(st, ctx, oracle, bulk, N, F, neg_th, odd):
-    """k_grain_bulk tile/stage shapes against the register-transpose kernel's cases: ragged
-    last tiles, ragged last warp, negative thresholds and non-reference state values
+def test_square_grain_bulk_variants(st, ctx, oracle, mode, N, F, neg_th, odd):
+    """The PLANAR kernels by planar_bulk (0 register transpose, 1 per-lane bulk copies, 2 tensor
+    TMA): ragged last tiles, ragged last warp, negative thresholds and non-reference state values
     (both take the literal two-branch form)."""
-    ctx.set_option("grain_bulk", bulk)
+    ctx.set_option("planar_bulk", mode)
     try:
         _square_grain_case(st, ctx, oracle, N, F, "PLANAR", neg_th, odd)
     finally:
-        ctx.set_option("grain_bulk", 5)
+        ctx.set_option("planar_bulk", 2)
 
 
 @pytest.mark.parametrize("gen", [0, 1, 2])

@@ -11,8 +11,8 @@ ncu --metrics gpu__time_duration.sum --clock-control none -c 700 --csv --log-fil
     python bench.py --steps 1 --warmup 1 > $O/bench_under_ncu.log 2>&1
 NCU="ncu --set full --clock-control none --import-source on -c 1"
 $NCU -k regex:k_pdm_v2_ws4 -s 2 -o $O/prof_pdm_v2_ws4 python tools/prof_pdm.py 131072 v2 > /dev/null 2>&1
-$NCU -k regex:k_grain_tma -s 1 -o $O/prof_grain_tma python tools/prof_one.py grain 1 > /dev/null 2>&1
-$NCU -k regex:k_grain_interleaved4 -s 1 -o $O/prof_grain_il4 python tools/prof_one.py grain_il 1 > /dev/null 2>&1
+$NCU -k regex:k_planar_tma -s 1 -o $O/prof_grain_tma python tools/prof_one.py grain 1 > /dev/null 2>&1
+$NCU -k regex:k_interleaved4 -s 1 -o $O/prof_grain_il4 python tools/prof_one.py grain_il 1 > /dev/null 2>&1
 $NCU -k regex:k_grain_mix3 -s 1 -o $O/prof_grain_mix3 python tools/prof_one.py gmix 1 > /dev/null 2>&1
 $NCU -k regex:k_xvoice_mix -s 1 -o $O/prof_xvoice_mix python tools/prof_one.py xvoice 1 > /dev/null 2>&1
 $NCU -k regex:k_voice_mix -s 1 -o $O/prof_voice_mix python tools/prof_one.py voice 1 > /dev/null 2>&1

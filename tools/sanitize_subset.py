@@ -8,7 +8,7 @@ import __graft_entry__ as ge
 import synth_tools_b200 as st
 from oracle import pyoracle as po
 
-ge.smoke()                       # k_pdm_v2_ws4 (static + dynamic schedule), k_voice_mix, k_grain_tma, graph_planar_tma (int and float graphs)
+ge.smoke()                       # k_pdm_v2_ws4 (static + dynamic schedule), k_voice_mix, k_planar_tma<GrainOp>, graph_planar_tma (int and float graphs)
 orc = po.Oracle()
 ctx = st.Context(0)
 rng = np.random.default_rng(1)
@@ -69,7 +69,7 @@ r = np.zeros((Nx, Fx, 2), np.float32)
 b.run(Fx, out=r)
 assert np.array_equal(r.view(np.uint32), raw.reshape(Nx, Fx, 2).view(np.uint32)), "xvoice raw"
 b.free()
-# square_grain mix (k_grain_mix3), interleaved square_grain (k_grain_interleaved4), graph interleaved4, graph scan, patcher
+# square_grain mix (k_grain_mix3), interleaved square_grain (k_interleaved4<GrainOp>), graph interleaved4, graph scan, patcher
 Ng, Fg = 4096, 64
 gs = np.zeros((Ng, 2), np.uint32); gs[:, 1] = rng.integers(0, 2**32, Ng, dtype=np.uint32)
 gp = np.zeros((Ng, 4), np.uint32); gp[:, 0] = rng.uniform(0.05, 0.5, Ng).astype(np.float32).view(np.uint32); gp[:, 1] = rng.integers(1 << 20, 1 << 26, Ng)
