@@ -118,7 +118,10 @@ enum cproc_cuda_proc {
     /* square_grain fed by a per-grain phasor (acc -> signed saw) and mixed
      * to stereo with dyadic pan gains k/64, integer mix in units of 2^-7.
      * state {float state; uint32 phase}; param {float threshold; uint32 inc;
-     * uint32 gl; uint32 gr}; out float [2][F]; mix int32 [2][F]. */
+     * uint32 gl; uint32 gr}; out float [2][F]; mix int32 [2][F].  Either
+     * may be NULL, not both.  With a mix bus attached (cproc_cuda_bus_attach)
+     * they receive the bus of ALL ranks: mix the summed int32 words, out
+     * (float)word * 2^-7. */
     CPROC_CUDA_SQUARE_GRAIN_MIX = 8,
     /* Extension voice (not in the reference): phasor -> Chamberlin SVF ->
      * linear AR envelope -> pan.  state {uint32 phase; float lp, bp, env;
@@ -413,7 +416,7 @@ int  cproc_cuda_bus_allreduce(cproc_cuda_bus *bus, int32_t *imix_dev, float *out
  * the context stream wait for that slot's last exchange. */
 int  cproc_cuda_bus_allreduce_begin(cproc_cuda_bus *bus, uint32_t slot, int32_t *imix_dev, float *out_dev, uint64_t count, uint32_t op, uint32_t scale);
 int  cproc_cuda_bus_wait(cproc_cuda_bus *bus, uint32_t slot);
-/* The exchange as the tail of the render kernel.  After _attach, cproc_cuda_run_dev on the batch (VOICE_BANK, XVOICE mix) renders the
+/* The exchange as the tail of the render kernel.  After _attach, cproc_cuda_run_dev on the batch (VOICE_BANK, XVOICE mix, SQUARE_GRAIN_MIX) renders the
  * shard's mix AND exchanges it in the same launch: the blocks that complete a piece of the local mix push it into every
  * peer's bus buffer, the last one publishes the flags.  io.mix / io.out then receive the bus of ALL ranks (reduced integer
  * words / scaled float), like after _allreduce.

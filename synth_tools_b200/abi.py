@@ -512,7 +512,8 @@ class Bus:
     IN_LAUNCH, PIPELINED = 1, 2
 
     def attach(self, batch, mode=1):
-        """The batch's render launch exchanges its mix itself (mode 1: reduce in the same launch, 2: beside the next one)."""
+        """The batch's render launch exchanges its mix itself (mode 1: reduce in the same launch, 2: beside the next one).
+        VOICE_BANK, XVOICE (mix only) and SQUARE_GRAIN_MIX batches."""
         self.ctx._ck(lib.cproc_cuda_bus_attach(self.h, batch.h, mode))
 
     def detach(self, batch):

@@ -252,8 +252,8 @@ int cproc_cuda_bus_attach(cproc_cuda_bus *bus, cproc_cuda_batch *batch, uint32_t
     if (bus->ctx != ctx) return cproc_set_err(ctx, CPROC_CUDA_EINVAL, "bus_attach: bus and batch belong to different contexts");
     if (!bus->connected) return cproc_set_err(ctx, CPROC_CUDA_ESTATE, "bus_attach: bus not connected (cproc_cuda_bus_connect)");
     const uint32_t proc = batch->cfg.proc;
-    if (proc != CPROC_CUDA_VOICE_BANK && proc != CPROC_CUDA_XVOICE)
-        return cproc_set_err(ctx, CPROC_CUDA_EINVAL, "bus_attach: only the voice bank and the xvoice mix exchange their bus in the render launch");
+    if (proc != CPROC_CUDA_VOICE_BANK && proc != CPROC_CUDA_XVOICE && proc != CPROC_CUDA_SQUARE_GRAIN_MIX)
+        return cproc_set_err(ctx, CPROC_CUDA_EINVAL, "bus_attach: only the voice bank, the xvoice mix and the square_grain mix exchange their bus in the render launch");
     batch->bus = bus; batch->bus_mode = mode;
     return 0;
 }

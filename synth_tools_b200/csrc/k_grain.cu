@@ -19,8 +19,11 @@
 //   alias out, as in Pd), and the tile is written back with 32 coalesced row stores.
 // k_grain_interleaved: the INTERLEAVED fallback, one grain per thread.
 // k_grain_mix: config C3b -- input from a per-grain phasor, integer stereo mix.
+//   k_grain_mix2 / k_grain_mix3 are its faster generations; all three take <BUS>: with
+//   a mix bus attached (cproc_cuda_bus_attach) the launch exchanges its mix itself.
 #include "common.cuh"
 #include "planar_bulk.cuh"
+#include "bus_fused.cuh"
 
 struct GrainParams {
     float *state;            // SoA [1][npad]
@@ -137,18 +140,53 @@ struct GrainMixParams {
     uint32_t *st;            // SoA [2][npad]: state (float bits), phase
     const uint32_t *prm;     // SoA [4][npad]: threshold (float bits), inc, gl, gr
     uint64_t npad, n, F;
-    int32_t *imix;           // [2][F], zeroed by the launcher
+    int32_t *imix;           // [2][F], zeroed by the launcher; with a bus: [2][F] + ticket, zero between launches
 };
+
+// With a mix bus attached (BUS) and pipelined (mode 2), block 0 runs the previous frame block's exchange and the
+// render blocks are 1..gridDim.x-1.  Block 0, not the last block: k_grain_mix is one thread per grain, many waves,
+// and a last block would start only after the last wave.  Returns false for the exchange block.
+template <bool BUS>
+__device__ __forceinline__ bool grain_render_block(const BusFused &bf, uint32_t &blk, uint32_t &nblk) {
+    blk = blockIdx.x; nblk = gridDim.x;
+    if (BUS && bf.mode == 2) {
+        if (blk == 0) { bus_exchange_block(bf); return false; }
+        --blk; --nblk;
+    }
+    return true;
+}
+
+// With a bus attached the render blocks accumulate into the batch's [2][F] accumulator (zero between launches), then
+// take a ticket; the last render block of the launch reads every word back with atomicExch(.., 0), which leaves the
+// accumulator zero for the next launch, emits it to the bus and completes the exchange (mode 1) or stages it (mode 2).
+// The kernels call it under `if constexpr (BUS)`: a plain `if` changes the register allocation of the BUS = false
+// instantiation, which is meant to stay the kernel without a bus, instruction for instruction.
+__device__ __forceinline__ void grain_bus_tail(int32_t *acc, uint64_t F, const BusFused &bf, uint32_t nblk) {
+    __shared__ uint32_t last_s;
+    uint32_t *ticket = (uint32_t *)(acc + 2 * F);
+    __threadfence();
+    __syncthreads();
+    if (threadIdx.x == 0) last_s = atomicAdd(ticket, 1u) == nblk - 1u;
+    __syncthreads();
+    if (!last_s) return;                      // (uniform over the block)
+    __threadfence();
+    for (uint64_t i = threadIdx.x; i < 2 * F; i += blockDim.x) bus_emit_word(bf, i, (uint32_t)atomicExch(acc + i, 0));
+    if (threadIdx.x == 0) *ticket = 0;
+    bus_participant_done(bf);
+}
 
 #define GMIX_BLOCK 256
 #define GMIX_CHUNK 32
-__global__ void __launch_bounds__(GMIX_BLOCK) k_grain_mix(const GrainMixParams p) {
+template <bool BUS>
+__global__ void __launch_bounds__(GMIX_BLOCK) k_grain_mix(const GrainMixParams p, const BusFused bf) {
     // Each lane keeps one grain in registers.  Left and right gains (0..64) are
     // packed into one word so one REDUX.SUM per frame reduces both channels
     // over the warp; warp sums are accumulated per block in shared memory and
     // flushed to the global integer mix once per chunk of frames.
     __shared__ int32_t acc[2][GMIX_CHUNK];
-    const uint64_t g = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    uint32_t blk, nblk;
+    if (!grain_render_block<BUS>(bf, blk, nblk)) return;
+    const uint64_t g = (uint64_t)blk * blockDim.x + threadIdx.x;
     const bool mine = g < p.n;
     const uint32_t lane = threadIdx.x & 31;
     float state = 0.0f, th = 0.0f;
@@ -186,6 +224,7 @@ __global__ void __launch_bounds__(GMIX_BLOCK) k_grain_mix(const GrainMixParams p
         __syncthreads();
     }
     if (mine) { p.st[g] = __float_as_uint(state); p.st[p.npad + g] = ph; }
+    if constexpr (BUS) grain_bus_tail(p.imix, p.F, bf, nblk);
 }
 
 // ---------------------------------------------------------------------------
@@ -260,10 +299,13 @@ __device__ __forceinline__ void gm2_load(GM2Grain &v, const GrainMix2Params &p, 
     v.lo = __ldg(p.lo + g); v.hi = __ldg(p.hi + g);
 }
 
-__global__ void __launch_bounds__(GM2_BLOCK) k_grain_mix2(const GrainMix2Params p) {
+template <bool BUS>
+__global__ void __launch_bounds__(GM2_BLOCK) k_grain_mix2(const GrainMix2Params p, const BusFused bf) {
     __shared__ int32_t sacc[2][GM2_CHUNK];
-    const uint64_t T = (uint64_t)gridDim.x * GM2_BLOCK;
-    const uint64_t tid = (uint64_t)blockIdx.x * GM2_BLOCK + threadIdx.x;
+    uint32_t blk, nblk;
+    if (!grain_render_block<BUS>(bf, blk, nblk)) return;
+    const uint64_t T = (uint64_t)nblk * GM2_BLOCK;
+    const uint64_t tid = (uint64_t)blk * GM2_BLOCK + threadIdx.x;
     const uint32_t lane = threadIdx.x & 31;
     const uint64_t n = p.g.n, npad = p.g.npad;
     for (uint64_t t0 = 0; t0 < p.g.F; t0 += GM2_CHUNK) {
@@ -313,6 +355,7 @@ __global__ void __launch_bounds__(GM2_BLOCK) k_grain_mix2(const GrainMix2Params 
         }
         __syncthreads();
     }
+    if constexpr (BUS) grain_bus_tail(p.g.imix, p.g.F, bf, nblk);
 }
 
 // ---------------------------------------------------------------------------
@@ -364,10 +407,13 @@ __device__ __forceinline__ void gm3_chunk(const GM3Grain &cur, uint32_t cols, in
     ph_out = ph;
 }
 
-__global__ void __launch_bounds__(GM3_BLOCK) k_grain_mix3(const GrainMix3Params p) {
+template <bool BUS>
+__global__ void __launch_bounds__(GM3_BLOCK) k_grain_mix3(const GrainMix3Params p, const BusFused bf) {
     __shared__ int32_t sacc[2][GM3_CHUNK];
-    const uint64_t T = (uint64_t)gridDim.x * GM3_BLOCK;
-    const uint64_t tid = (uint64_t)blockIdx.x * GM3_BLOCK + threadIdx.x;
+    uint32_t blk, nblk;
+    if (!grain_render_block<BUS>(bf, blk, nblk)) return;
+    const uint64_t T = (uint64_t)nblk * GM3_BLOCK;
+    const uint64_t tid = (uint64_t)blk * GM3_BLOCK + threadIdx.x;
     const uint32_t lane = threadIdx.x & 31;
     const uint64_t n = p.g.n, npad = p.g.npad;
     for (uint64_t t0 = 0; t0 < p.g.F; t0 += GM3_CHUNK) {
@@ -407,6 +453,7 @@ __global__ void __launch_bounds__(GM3_BLOCK) k_grain_mix3(const GrainMix3Params 
         }
         __syncthreads();
     }
+    if constexpr (BUS) grain_bus_tail(p.g.imix, p.g.F, bf, nblk);
 }
 
 __global__ void k_imix_to_float(const int32_t *imix, float *mix, uint64_t count, float scale) {
@@ -419,17 +466,30 @@ int launch_square_grain_mix(cproc_cuda_batch *b, uint64_t F, const cproc_cuda_io
     if (!io->out && !io->mix) return cproc_set_err(ctx, CPROC_CUDA_EINVAL, "square_grain_mix: out and mix are both NULL");
     if (F == 0) return 0;
     int32_t *imix = (int32_t *)io->mix;
-    if (!imix) {
-        size_t need = sizeof(int32_t) * 2 * F;
-        if (b->cap_mix < need) {
-            if (b->d_mix) cudaFree(b->d_mix);
-            b->d_mix = nullptr; b->cap_mix = 0;
-            CK(ctx, cudaMalloc(&b->d_mix, need));
-            b->cap_mix = need;
+    if (b->bus) {
+        // the launch exchanges its mix itself: a [2][F] accumulator + ticket that every launch leaves zero, no memset
+        const size_t need = sizeof(int32_t) * (2 * F + 1);
+        if (b->cap_acc < need) {
+            if (b->d_acc) cudaFree(b->d_acc);
+            b->d_acc = nullptr; b->cap_acc = 0;
+            CK(ctx, cudaMalloc(&b->d_acc, need));
+            CK(ctx, cudaMemsetAsync(b->d_acc, 0, need, ctx->stream));   // once
+            b->cap_acc = need;
         }
-        imix = (int32_t *)b->d_mix;
+        imix = (int32_t *)b->d_acc;
+    } else {
+        if (!imix) {
+            size_t need = sizeof(int32_t) * 2 * F;
+            if (b->cap_mix < need) {
+                if (b->d_mix) cudaFree(b->d_mix);
+                b->d_mix = nullptr; b->cap_mix = 0;
+                CK(ctx, cudaMalloc(&b->d_mix, need));
+                b->cap_mix = need;
+            }
+            imix = (int32_t *)b->d_mix;
+        }
+        CK(ctx, cudaMemsetAsync(imix, 0, sizeof(int32_t) * 2 * F, ctx->stream));
     }
-    CK(ctx, cudaMemsetAsync(imix, 0, sizeof(int32_t) * 2 * F, ctx->stream));
     GrainMixParams p;
     p.st = b->d_state; p.prm = b->d_param; p.npad = b->npad; p.n = b->n; p.F = F; p.imix = imix;
     if (b->aux_dirty) {                                   // integer thresholds, once per parameter upload
@@ -444,31 +504,42 @@ int launch_square_grain_mix(cproc_cuda_batch *b, uint64_t F, const cproc_cuda_io
         b->aux_weird = h;
         b->aux_dirty = false;
     }
+    // one pusher: the last render block of the launch; the bus writes io->mix (int32) and io->out ((float)x * 2^-7)
+    BusFused bf;
+    int rc = cproc_bus_fused_begin(b, &bf, 2 * F, 0u, 3u, 1u, (int32_t *)io->mix, (float *)io->out);
+    if (rc) return rc;
+    // a pipelined bus adds block 0, which completes the previous frame block's exchange; the capped grids below keep
+    // it a free slot from the start
+    const uint32_t xb = bf.world && bf.mode == 2 ? 1u : 0u;
+#define GRAIN_MIX_LAUNCH(K, blocks, BLK, q) do { \
+        if (bf.world) K<true><<<(unsigned)(blocks) + xb, BLK, 0, ctx->stream>>>(q, bf); \
+        else K<false><<<(unsigned)(blocks), BLK, 0, ctx->stream>>>(q, bf); } while (0)
     if (ctx->grain_mix2 >= 2 && !b->aux_weird) {
         GrainMix3Params q;
         q.g = p; q.lo = (const int32_t *)b->d_aux; q.hi = q.lo + b->npad; q.pk = q.lo + 2 * b->npad;
         uint64_t blocks = ceil_div_u64(p.n, GM3_BLOCK);
-        const uint64_t cap = (uint64_t)ctx->n_sm * (uint64_t)ctx->grain_blocks_per_sm;
+        const uint64_t cap = (uint64_t)ctx->n_sm * (uint64_t)ctx->grain_blocks_per_sm - xb;
         if (blocks > cap) blocks = cap;
         const uint64_t min_blocks = ceil_div_u64(p.n, (uint64_t)GM3_BLOCK * 500);   // packed 16-bit bus fields: <= 500 grains per thread
         if (blocks < min_blocks) blocks = min_blocks;
-        k_grain_mix3<<<(unsigned)blocks, GM3_BLOCK, 0, ctx->stream>>>(q);
+        GRAIN_MIX_LAUNCH(k_grain_mix3, blocks, GM3_BLOCK, q);
         CK_LAUNCH(ctx, "k_grain_mix3");
     } else if (ctx->grain_mix2 && !(b->aux_weird & 1u)) {
         GrainMix2Params q;
         q.g = p; q.lo = (const int32_t *)b->d_aux; q.hi = (const int32_t *)b->d_aux + b->npad;
         uint64_t blocks = ceil_div_u64(p.n, GM2_BLOCK);
-        const uint64_t cap = (uint64_t)ctx->n_sm * (uint64_t)ctx->grain_blocks_per_sm;
+        const uint64_t cap = (uint64_t)ctx->n_sm * (uint64_t)ctx->grain_blocks_per_sm - xb;
         if (blocks > cap) blocks = cap;
         const uint64_t min_blocks = ceil_div_u64(p.n, (uint64_t)GM2_BLOCK * 500);   // packed 16-bit bus fields: <= 500 grains per thread
         if (blocks < min_blocks) blocks = min_blocks;
-        k_grain_mix2<<<(unsigned)blocks, GM2_BLOCK, 0, ctx->stream>>>(q);
+        GRAIN_MIX_LAUNCH(k_grain_mix2, blocks, GM2_BLOCK, q);
         CK_LAUNCH(ctx, "k_grain_mix2");
     } else {
-        k_grain_mix<<<(unsigned)ceil_div_u64(p.n, GMIX_BLOCK), GMIX_BLOCK, 0, ctx->stream>>>(p);
+        GRAIN_MIX_LAUNCH(k_grain_mix, ceil_div_u64(p.n, GMIX_BLOCK), GMIX_BLOCK, p);
         CK_LAUNCH(ctx, "k_grain_mix");
     }
-    if (io->out) {
+#undef GRAIN_MIX_LAUNCH
+    if (io->out && !bf.world) {
         k_imix_to_float<<<(unsigned)ceil_div_u64(2 * F, 256), 256, 0, ctx->stream>>>(imix, (float *)io->out, 2 * F, 0x1p-7f);
         CK_LAUNCH(ctx, "k_imix_to_float");
     }

@@ -10,9 +10,12 @@ memory, reduce and float scale fused, (C) the exchange fused into the render lau
 (cproc_cuda_bus_attach mode 1: reduce at the end of the same launch), (D) the same, pipelined
 (mode 2: the reduce of block k beside the render of block k+1).  All must equal the
 single-device oracle bit for bit.  Prints one JSON line per measurement (rank 0).
+The C4 extension voices (float bus) and the C3b square_grain mix (1 Mi grains x 256-frame
+blocks, integer bus in units of 2^-7) get the same treatment in their own sections.
 --check-only: parity checks at reduced sizes, no timing (tests/test_gpu_multi.py)."""
 import json
 import os
+import subprocess
 import sys
 
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
@@ -305,12 +308,148 @@ def xvoice_check_and_timing(N_check, N, F, reps=20):
     return ok, res
 
 
+def grain_records(N, seed):
+    """state, threshold, phase, inc, gl, gr of N grains (the same on every rank)"""
+    r = np.random.default_rng(seed)
+    state = r.choice(np.array([0.0, 0.5, -0.5], np.float32), N)
+    th = r.uniform(0.05, 0.5, N).astype(np.float32)
+    phase = r.integers(0, 2**32, N, dtype=np.uint32)
+    inc = tab[r.integers(36, 97, N)]
+    gl = r.integers(0, 65, N).astype(np.uint8)
+    return state, th, phase, inc, gl, (64 - gl).astype(np.uint8)
+
+
+def grain_batch(g, lo, hi):
+    state, th, phase, inc, gl, gr = (x[lo:hi] for x in g)
+    b = ctx.batch(st.SQUARE_GRAIN_MIX, hi - lo)
+    s_rec = np.zeros((hi - lo, 2), np.uint32); s_rec[:, 0] = state.view(np.uint32); s_rec[:, 1] = phase
+    p_rec = np.zeros((hi - lo, 4), np.uint32); p_rec[:, 0] = th.view(np.uint32); p_rec[:, 1] = inc; p_rec[:, 2] = gl; p_rec[:, 3] = gr
+    b.upload_state(s_rec); b.upload_param(p_rec)
+    return b
+
+
+def grain_check(N, F, K=6):
+    """C3b: K consecutive blocks of the sharded grain mix, the bus formed by the separate bus kernel and by the exchange fused
+    into the render launch (modes 1 and 2), each compared on every rank with the single-device oracle."""
+    g = grain_records(N, 77)
+    lo, hi = shard.shard_range(N, rank, world)
+    ga = tuple(x.copy() for x in g)
+    wants = [orc.square_grain_mix_run(*ga, N, F) for _ in range(K)]
+
+    def same(imix, out, k):
+        return np.array_equal(imix.cpu().numpy().reshape(2, F), wants[k][0]) and \
+            np.array_equal(out.cpu().numpy().reshape(2, F).view(np.uint32), wants[k][1].view(np.uint32))
+
+    bus = shard.connect_bus(st.Bus(ctx, 4096, world, rank))
+    mixes = [torch.zeros(2 * F, dtype=torch.int32, device=dev) for _ in range(K)]
+    outs = [torch.zeros(2 * F, dtype=torch.float32, device=dev) for _ in range(K)]
+    b = grain_batch(g, lo, hi)
+    for k in range(K):                                    # the separate bus kernel after each render
+        b.run_dev(F, mix=mixes[k].data_ptr())
+        bus.allreduce(mixes[k].data_ptr(), 2 * F, out_dev=outs[k].data_ptr(), scale=st.Bus.SCALE_GRAIN)
+    torch.cuda.synchronize()
+    ok_sep = bus.status() == 0 and all(same(mixes[k], outs[k], k) for k in range(K))
+    b.free()
+    ok_f = []
+    for bus_mode in (1, 2):
+        b = grain_batch(g, lo, hi)
+        bus.attach(b, bus_mode)
+        for m, o in zip(mixes, outs):
+            m.zero_(); o.zero_()
+        for k in range(K):
+            b.run_dev(F, mix=mixes[k].data_ptr(), out=outs[k].data_ptr())
+        bus.flush()
+        torch.cuda.synchronize()
+        ok_f.append(bus.status() == 0 and all(same(mixes[k], outs[k], k) for k in range(K)))
+        bus.detach(b)
+        b.free()
+    bus.destroy()
+    t = torch.tensor([int(ok_sep), int(ok_f[0]), int(ok_f[1])], device=dev)
+    dist.all_reduce(t, op=dist.ReduceOp.MIN)
+    return [bool(x.item()) for x in t]
+
+
+def grain_timing(N, F, reps=400, rounds=3):
+    """C3b at full size: ms per 256-frame block, CUDA events, max over ranks; each form timed `rounds` times, in turn."""
+    g = grain_records(N, 78)
+    lo, hi = shard.shard_range(N, rank, world)
+    b = grain_batch(g, lo, hi)
+    bus = shard.connect_bus(st.Bus(ctx, 4096, world, rank))
+    mixes = [torch.zeros(2 * F, dtype=torch.int32, device=dev) for _ in range(2)]
+    outs = [torch.zeros(2 * F, dtype=torch.float32, device=dev) for _ in range(2)]
+    mix4 = torch.zeros(8 * F, dtype=torch.int32, device=dev)
+    out4 = torch.zeros(8 * F, dtype=torch.float32, device=dev)
+    k = [0]
+
+    def render_only():
+        b.run_dev(F, mix=mixes[0].data_ptr(), out=outs[0].data_ptr())
+
+    def separate_bus():                                   # today's form: the bus kernel on the bus's stream, overlapped
+        s = k[0] & 1
+        k[0] += 1
+        bus.wait(s)
+        b.run_dev(F, mix=mixes[s].data_ptr(), out=outs[s].data_ptr())
+        bus.begin(s, mixes[s].data_ptr(), 2 * F, out_dev=outs[s].data_ptr(), scale=st.Bus.SCALE_GRAIN)
+
+    def fused():
+        s = k[0] & 1
+        k[0] += 1
+        b.run_dev(F, mix=mixes[s].data_ptr(), out=outs[s].data_ptr())
+
+    def fused_k4():                                       # four frame blocks per launch, one exchange of [2][4 x 256]
+        b.run_dev(4 * F, mix=mix4.data_ptr(), out=out4.data_ptr())
+
+    forms = (("render_only", 0, render_only, 1), ("separate_bus_kernel_overlapped", 0, separate_bus, 1), ("fused_in_launch", 1, fused, 1),
+             ("fused_pipelined", 2, fused, 1), ("fused_pipelined_4_blocks_per_launch", 2, fused_k4, 4))
+    res = {name: [] for name, _, _, _ in forms}
+    for _ in range(rounds):
+        for name, mode, fn, per in forms:
+            if mode:
+                bus.attach(b, mode)
+            else:
+                bus.detach(b)
+            for _ in range(10):
+                fn()
+            bus.wait(0); bus.wait(1); bus.flush()
+            dist.barrier(); torch.cuda.synchronize()
+            n = max(1, reps // per)
+            e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+            e0.record(stream)
+            for _ in range(n):
+                fn()
+            bus.wait(0); bus.wait(1); bus.flush()
+            e1.record(stream)
+            dist.barrier(); torch.cuda.synchronize()
+            t = torch.tensor([e0.elapsed_time(e1) / (n * per)], device=dev, dtype=torch.float64)
+            dist.all_reduce(t, op=dist.ReduceOp.MAX)
+            res[name].append(float(t.item()))
+    ok = bus.status() == 0
+    bus.detach(b)
+    bus.destroy(); b.free()
+    return res, ok
+
+
+def card():
+    """name and power limit of this rank's GPU, read in the same run as the measurement"""
+    try:
+        r = subprocess.run(["nvidia-smi", "-i", str(torch.cuda.current_device()), "--query-gpu=power.limit,clocks.max.sm", "--format=csv,noheader"],
+                           capture_output=True, text=True, timeout=30)
+        limit = r.stdout.strip() or None
+    except (OSError, subprocess.SubprocessError):
+        limit = None
+    return {"name": torch.cuda.get_device_name(dev), "power_limit_and_max_sm_clock": limit}
+
+
 CHECK_ONLY = "--check-only" in sys.argv
 for mode in (0, 1):
     a, bb, c1, c2 = check(256 * 1024 + 77, 512, mode)
     if rank == 0:
         print(json.dumps({"check": "voice bank mix bus, mode %d" % mode, "n_gpus": world, "nccl_bit_exact": a, "peer_bus_bit_exact": bb,
                           "fused_in_launch_bit_exact": c1, "fused_pipelined_bit_exact": c2}), flush=True)
+sep, f1, f2 = grain_check(256 * 1024 + 77, 256)
+if rank == 0:
+    print(json.dumps({"check": "square_grain mix bus", "n_gpus": world, "peer_bus_bit_exact": sep, "fused_in_launch_bit_exact": f1,
+                      "fused_pipelined_bit_exact": f2}), flush=True)
 if CHECK_ONLY:
     okx, detail = xvoice_check_and_timing(64 * 1024 + 5, 0, 512)
     if rank == 0:
@@ -332,5 +471,12 @@ if rank == 0:
     print(json.dumps({"config": "C4 poly voice 4 Mi voices x 512 frames sharded over %d GPUs, float stereo mix bus" % world, "n_gpus": world,
                       "float_bus_within_tolerance_and_identical_on_all_ranks": bool(okx), "ms_per_block": resx,
                       "voice_samples_per_s": {k: N * F / (v * 1e-3) for k, v in resx.items()}}), flush=True)
+resg, okg = grain_timing(1024 * 1024, 256)
+if rank == 0:
+    N, F = 1024 * 1024, 256
+    med = {k: float(np.median(v)) for k, v in resg.items()}
+    print(json.dumps({"config": "C3b square_grain mix 1 Mi grains x 256-frame blocks sharded over %d GPUs, int32 mix bus" % world, "n_gpus": world, "bus_ok": okg,
+                      "card": card(), "ms_per_block": med, "ms_per_block_rounds": resg,
+                      "grain_samples_per_s": {k: N * F / (v * 1e-3) for k, v in med.items()}}), flush=True)
 ctx.close()
 dist.destroy_process_group()
