@@ -34,7 +34,8 @@ def _note_incs(orc, n, lo, hi):
 
 
 def test_c2_pdm_v2_full_launch_shape(st, ctx, oracle):
-    """65,536 channels x 65,536 ticks (one launch of the headline bench), banks of 3, a setpoint
+    """65,536 channels x 65,536 ticks (half of one 131,072-tick launch of the headline bench, from count 0;
+    the whole step, launch for launch: tests/test_gpu_bench_shapes.py), banks of 3, a setpoint
     row every 4096 ticks.  (1) the oracle on banks 0..31, 10,000..10,031 and the last 32 banks
     (with the ragged last bank) reproduces their duty bytes, state and PRNG words exactly;
     (2) k_pdm_v2_ws4 with 128-tick and with 64-tick dither batches and the plain thread-per-bank kernel
