@@ -121,7 +121,10 @@ enum cproc_cuda_proc {
      * uint32 gl; uint32 gr}; out float [2][F]; mix int32 [2][F].  Either
      * may be NULL, not both.  With a mix bus attached (cproc_cuda_bus_attach)
      * they receive the bus of ALL ranks: mix the summed int32 words, out
-     * (float)word * 2^-7. */
+     * (float)word * 2^-7.
+     * gl, gr <= 64: upload_param returns CPROC_CUDA_EINVAL above 64.
+     * Every float state acts and comes back as in the reference (a NaN state never flips
+     * and adds 0); a state other than +-0, +-0.5 selects a slower kernel until the next upload. */
     CPROC_CUDA_SQUARE_GRAIN_MIX = 8,
     /* Extension voice (not in the reference): phasor -> Chamberlin SVF ->
      * linear AR envelope -> pan.  state {uint32 phase; float lp, bp, env;
@@ -462,7 +465,8 @@ int  cproc_cuda_timer_stop(cproc_cuda_ctx *ctx, float *elapsed_ms);
  *   pdm_v1_chains    1/2  [2]  PDM v1: PRNG chains per lane
  *   pdm_block, pdm_tpb [2: auto; 1 thread per bank when bank_size <= 4; 0 thread per channel], pdm_persist, pdm_warps_per_smsp   plain PDM kernels, PDM v1 schedule
  *   xvoice_mix2      0/1  [1]  XVOICE mix-only render: voice pairs on the packed fp32 pipe (FFMA2) with state tiles in shared
- *                              memory; 0 = the scalar kernel (state through L2 once per 32-frame chunk)
+ *                              memory; 0 = the scalar kernel (state through L2 once per 32-frame chunk).  Known deviation of 1:
+ *                              it runs the filter on -lp, so where lp + f*bp cancels exactly the state holds lp = -0, not +0
  *   xvoice_mix2_blocks 0..3 [0] its resident blocks per SM (0 = chosen from the voice count)
  *   xvoice_chunk [0 = auto], xvoice_groups 0..8 [0 = one group], xvoice_closed 0/1 [1]
  *                              XVOICE_SCAN: frames per time chunk, variant groups, closed-form zero-state pass

@@ -250,6 +250,12 @@ int cproc_cuda_free(cproc_cuda_batch *b) {
 size_t cproc_cuda_state_bytes(const cproc_cuda_batch *b) { return b ? 4u * b->state_words : 0; }
 size_t cproc_cuda_param_bytes(const cproc_cuda_batch *b) { return b ? 4u * b->param_words : 0; }
 
+// k_grain_mix2 / k_grain_mix3 carry a grain's trigger state as -1 / 0 / +1 and write back +-0.5; the reference keeps any
+// other float (0.3, a subnormal, +-inf; a NaN state never flips and adds 0 to the mix).  Such a state needs k_grain_mix.
+static bool grain_state_odd(uint32_t w) {
+    return w != 0u && w != 0x80000000u && w != 0x3F000000u && w != 0xBF000000u;
+}
+
 // AoS (reference struct layout, any stride) <-> SoA rows on the device.
 static int aos_to_dev(cproc_cuda_batch *b, uint32_t *d_rows, uint32_t words, const void *aos, size_t stride) {
     cproc_cuda_ctx *ctx = b->ctx;
@@ -263,6 +269,10 @@ static int aos_to_dev(cproc_cuda_batch *b, uint32_t *d_rows, uint32_t words, con
         uint32_t rec[5 * CPROC_CUDA_GRAPH_MAX_NODES + 8];
         memcpy(rec, src + i * stride, 4u * words);
         for (uint32_t w = 0; w < words; ++w) soa[(size_t)w * b->npad + i] = rec[w];
+    }
+    if (d_rows == b->d_state && b->cfg.proc == CPROC_CUDA_SQUARE_GRAIN_MIX) {
+        b->grain_odd_state = false;
+        for (uint64_t i = 0; i < b->n; ++i) b->grain_odd_state |= grain_state_odd(soa[i]);
     }
     CK(ctx, cudaSetDevice(ctx->device));
     CK(ctx, cudaMemcpyAsync(d_rows, soa.data(), sizeof(uint32_t) * soa.size(), cudaMemcpyHostToDevice, ctx->stream));
@@ -278,6 +288,16 @@ int cproc_cuda_upload_state(cproc_cuda_batch *b, const void *aos, size_t stride)
 int cproc_cuda_upload_param(cproc_cuda_batch *b, const void *aos, size_t stride) {
     if (!b) return cproc_set_err(nullptr, CPROC_CUDA_EINVAL, "upload_param: batch is NULL");
     if (b->param_words == 0) return cproc_set_err(b->ctx, CPROC_CUDA_EINVAL, "upload_param: processor has no param record");
+    if (b->cfg.proc == CPROC_CUDA_SQUARE_GRAIN_MIX && aos && (stride == 0 || stride >= 4u * b->param_words)) {
+        // pan gains k/64: the mix kernels pack both channels of up to 500 grains into 16-bit halves
+        const size_t s = stride ? stride : 4u * b->param_words;
+        for (uint64_t i = 0; i < b->n; ++i) {
+            uint32_t g[2];
+            memcpy(g, (const uint8_t *)aos + i * s + 8, sizeof(g));
+            if (g[0] > 64 || g[1] > 64)
+                return cproc_set_err(b->ctx, CPROC_CUDA_EINVAL, "upload_param: square_grain_mix grain %llu: gains %u, %u (0..64)", (unsigned long long)i, g[0], g[1]);
+        }
+    }
     b->aux_dirty = true;
     return aos_to_dev(b, b->d_param, b->param_words, aos, stride);
 }
@@ -567,6 +587,10 @@ int cproc_cuda_run_period(cproc_cuda_batch *b, uint64_t F, const cproc_cuda_io *
     uint8_t *rec = (uint8_t *)state_aos;
     for (uint64_t i = 0; i < b->n; ++i)
         for (uint32_t w = 0; w < words; ++w) memcpy(b->st_h + (size_t)w * b->npad + i, rec + i * stride + 4u * w, 4);
+    if (b->cfg.proc == CPROC_CUDA_SQUARE_GRAIN_MIX) {
+        b->grain_odd_state = false;
+        for (uint64_t i = 0; i < b->n; ++i) b->grain_odd_state |= grain_state_odd(b->st_h[i]);
+    }
     CK(ctx, cudaMemcpyAsync(b->d_state, b->st_h, bytes, cudaMemcpyHostToDevice, ctx->stream));
     b->ride_state = true;
     const int rc = cproc_cuda_run(b, F, io);               // ends with the records' D2H copy and the period's one sync

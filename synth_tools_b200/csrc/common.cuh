@@ -87,6 +87,7 @@ struct cproc_cuda_batch {
     size_t cap_in = 0, cap_in2 = 0, cap_ctl = 0, cap_out = 0, cap_mix = 0;
     void *d_out2 = nullptr; size_t cap_out2 = 0;   // second slab for run_stream
     uint32_t *d_aux = nullptr; bool aux_dirty = true; uint32_t aux_weird = 0;   // derived parameter rows (grain mix integer thresholds)
+    bool grain_odd_state = false;           // grain mix: a state uploaded outside {+-0, +-0.5} (k_grain_mix until the next upload)
     void *d_scratch = nullptr; size_t cap_scratch = 0;   // per-chunk start-state tables (XVOICE_SCAN)
     uint32_t *d_acc = nullptr; size_t cap_acc = 0;       // voice bank: integer accumulators of a bus split over tiles + tickets; all zero between launches
     unsigned long long *d_flags = nullptr;         // persistent-kernel progress words

@@ -239,8 +239,8 @@ __global__ void __launch_bounds__(GMIX_BLOCK) k_grain_mix(const GrainMixParams p
 //    chunk one after the other; the state machine output m in {-1, 0, +1} enters the
 //    bus as one IMAD (acc += m * pk).  One warp reduction per frame per chunk instead
 //    of one per grain-sample.
-// State on the device stays the reference float (0, +0.5, -0.5); other magnitudes are
-// treated by their sign, as the integer mix always did, and come back as +-0.5.
+// This generation and the third write back only the reference's states (+-0, +-0.5): a
+// batch with any other state uploaded (grain_odd_state, abi.cu) runs k_grain_mix.
 __global__ void k_grain_thresholds(const uint32_t *prm, uint64_t n, uint64_t npad, int32_t *lo, int32_t *hi, int32_t *pk, uint32_t *weird) {
     const uint64_t g = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (g >= n) return;
@@ -514,7 +514,7 @@ int launch_square_grain_mix(cproc_cuda_batch *b, uint64_t F, const cproc_cuda_io
 #define GRAIN_MIX_LAUNCH(K, blocks, BLK, q) do { \
         if (bf.world) K<true><<<(unsigned)(blocks) + xb, BLK, 0, ctx->stream>>>(q, bf); \
         else K<false><<<(unsigned)(blocks), BLK, 0, ctx->stream>>>(q, bf); } while (0)
-    if (ctx->grain_mix2 >= 2 && !b->aux_weird) {
+    if (ctx->grain_mix2 >= 2 && !b->aux_weird && !b->grain_odd_state) {
         GrainMix3Params q;
         q.g = p; q.lo = (const int32_t *)b->d_aux; q.hi = q.lo + b->npad; q.pk = q.lo + 2 * b->npad;
         uint64_t blocks = ceil_div_u64(p.n, GM3_BLOCK);
@@ -524,7 +524,7 @@ int launch_square_grain_mix(cproc_cuda_batch *b, uint64_t F, const cproc_cuda_io
         if (blocks < min_blocks) blocks = min_blocks;
         GRAIN_MIX_LAUNCH(k_grain_mix3, blocks, GM3_BLOCK, q);
         CK_LAUNCH(ctx, "k_grain_mix3");
-    } else if (ctx->grain_mix2 && !(b->aux_weird & 1u)) {
+    } else if (ctx->grain_mix2 && !(b->aux_weird & 1u) && !b->grain_odd_state) {
         GrainMix2Params q;
         q.g = p; q.lo = (const int32_t *)b->d_aux; q.hi = (const int32_t *)b->d_aux + b->npad;
         uint64_t blocks = ceil_div_u64(p.n, GM2_BLOCK);
