@@ -77,7 +77,23 @@ enum cproc_cuda_proc {
      * cproc_output statements [inst][n_outputs][F].  A graph that reads no
      * input[] (a free-running phasor_f voice) has n_inputs == 0 and in == NULL.
      * param record: the nodes' param structs concatenated in ANF order (only the
-     * extension processors have one, see the node kinds below). */
+     * extension processors have one, see the node kinds below).
+     * mix (or NULL): the bus mix of every output, 32-bit words [bus][n_outputs][F], bus = instance /
+     * cfg.voices_per_bus (0: every instance on one bus); out may then be NULL (no per-instance stream is
+     * written), and with both set out holds what an out-only run writes.  Output q is a float when its
+     * node kind outputs a float (whichever of cproc_output / cproc_output_f named it): summed in binary32,
+     * one __fadd_rn rounding per add, no flush to zero; a w output is summed mod 2^32.  Summation order
+     * (part of the contract, so results are bit-reproducible): a balanced pairwise tree over the bus's
+     * instances in index order -- the instance count padded to a power of two with -0.0f (0 for w; adding
+     * -0 is an exact identity, so a one-instance bus gives its output), level 1 adds instances (2m, 2m+1),
+     * level 2 those pair sums, and so on.  The tree depends on the bus's instance count only: not on F,
+     * on how frames are split over calls, on the layout or on any cproc_cuda_set_option value.  With n
+     * instances on one bus, |mix - exact sum| <= gamma_d * sum |out|, d = ceil(log2 n), gamma_d = d u /
+     * (1 - d u), u = 2^-24.  A multi-GPU host all-reduces the mix with cproc_cuda_bus_allreduce, op 2 when
+     * every output is a float, op 0 when every output is a w.  The run call returns CPROC_CUDA_EINVAL with
+     * mix set for voices_per_bus neither 0 nor a multiple of 32, for cfg.mode = CPROC_CUDA_GRAPH_SCAN and
+     * for the TILED layout; there is no mix in cproc_cuda_run_stream or cproc_cuda_patch_tick, and
+     * cproc_cuda_bus_attach does not take GRAPH batches. */
     CPROC_CUDA_GRAPH = 1,
     /* pdmK_update, K = cfg.order (pdm.h).  state record: struct pdmK.
      * param record: {uint32 input} used when in == NULL.  in: uint32
@@ -243,7 +259,7 @@ typedef struct {
     uint32_t ctl_div_log;     /* CONTROL_DIV_LOG = 12 (mod_pdm_pwm.c:76)     */
     /* voice bank */
     uint32_t mode;            /* CPROC_CUDA_MIX_* / CPROC_CUDA_XVOICE_*      */
-    uint64_t voices_per_bus;  /* 0 = all instances on one bus                */
+    uint64_t voices_per_bus;  /* 0 = all instances on one bus (voice bank, graph mix) */
     /* graph */
     const cproc_cuda_node *nodes;
     uint32_t n_nodes, n_inputs, out_node;

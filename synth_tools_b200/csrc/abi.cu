@@ -207,6 +207,7 @@ int cproc_cuda_alloc(cproc_cuda_ctx *ctx, const cproc_cuda_config *cfg, uint64_t
         if (b->cfg.voices_per_bus == 0 || b->cfg.voices_per_bus > n) b->cfg.voices_per_bus = n;
         b->n_bus = ceil_div_u64(n, b->cfg.voices_per_bus);
     }
+    if (c.proc == CPROC_CUDA_GRAPH) b->n_bus = c.voices_per_bus == 0 ? 1 : ceil_div_u64(n, c.voices_per_bus);   // io.mix checks the value
     int rc = 0;
     do {
         if ((rc = cproc_check(ctx, cudaMalloc(&b->d_state, sizeof(uint32_t) * sw * b->npad), "cudaMalloc(state)"))) break;
@@ -359,7 +360,8 @@ int cproc_io_bytes(const cproc_cuda_batch *b, uint64_t F, const cproc_cuda_io *i
     memset(s, 0, sizeof(*s));
     switch (c.proc) {
     case CPROC_CUDA_GRAPH:
-        s->in = 4 * n * c.n_inputs * F; s->in2 = io->in2 ? 4 * n * F : 0; s->out = 4 * n * (c.n_outputs ? c.n_outputs : 1) * F; break;
+        s->in = 4 * n * c.n_inputs * F; s->in2 = io->in2 ? 4 * n * F : 0; s->out = io->out || !io->mix ? 4 * n * (c.n_outputs ? c.n_outputs : 1) * F : 0;
+        s->mix = io->mix ? 4 * b->n_bus * (c.n_outputs ? c.n_outputs : 1) * F : 0; break;
     case CPROC_CUDA_PDM:
         s->in = io->in ? 4 * n * F : 0; s->in2 = io->in2 ? 4 * F : 0; s->out = 4 * n * F; break;
     case CPROC_CUDA_PDM_V1:
@@ -441,9 +443,12 @@ int cproc_cuda_run(cproc_cuda_batch *b, uint64_t F, const cproc_cuda_io *io) {
     // in bulk -- the PLANAR staging kernels (one PCIe round trip per tile) and the voice bank's coalesced stores.  The
     // scalar fallbacks read a word per tick: over PCIe that is a round trip per tick.  An integer mix bus may be
     // accumulated with atomics: device memory only.
+    // The graph mix kernel reads and writes per instance and frame: only a mix-only render without input streams qualifies
+    // (its group sums go to the batch's device scratch, the bus mix straight to the staging).
     const bool zc_ok = io->layout == CPROC_CUDA_PLANAR && ctx->planar_bulk >= 1 &&
         (proc == CPROC_CUDA_VOICE_BANK ? io->mix == nullptr
          : proc == CPROC_CUDA_PWM ? F % 16 == 0
+         : proc == CPROC_CUDA_GRAPH && io->mix ? !io->in && !io->in2 && !io->out
          : F % 4 == 0);
     // run_graph 3: no graph and no copies -- direct launches on the pinned staging (one launch + one sync per period)
     if (ctx->run_graph >= 3 && graphable && zc_ok && sz.in + sz.in2 + sz.ctl + sz.out + sz.mix <= (64u << 10)) {

@@ -58,8 +58,8 @@ struct cproc_graph_jit {
     int state = 0;
     std::vector<char> cubin;
     cudaLibrary_t lib = nullptr;
-    cudaKernel_t k_il = nullptr, k_il4 = nullptr, k_pl = nullptr, k_ps = nullptr, k_pt = nullptr;
-    uint32_t pl_smem = 0, pl_block = 0, pt_smem = 0;
+    cudaKernel_t k_il = nullptr, k_il4 = nullptr, k_pl = nullptr, k_ps = nullptr, k_pt = nullptr, k_mix = nullptr;
+    uint32_t pl_smem = 0, pl_block = 0, pt_smem = 0, mix_warps = 0;   // mix_warps: block of the bus-mix kernel graph_mix, in warps
 };
 
 struct cproc_cuda_bus;
@@ -73,7 +73,7 @@ struct cproc_cuda_batch {
     uint64_t n = 0;                         // instances
     uint64_t npad = 0;                      // SoA row length (>= n)
     uint64_t n_banks = 0;
-    uint64_t n_bus = 0;
+    uint64_t n_bus = 0;                     // voice bank / graph mix: buses of cfg.voices_per_bus instances
     uint32_t state_words = 0, param_words = 0;
     uint32_t *d_state = nullptr;            // [state_words][npad]
     uint32_t *d_param = nullptr;            // [param_words][npad]
@@ -88,7 +88,7 @@ struct cproc_cuda_batch {
     void *d_out2 = nullptr; size_t cap_out2 = 0;   // second slab for run_stream
     uint32_t *d_aux = nullptr; bool aux_dirty = true; uint32_t aux_weird = 0;   // derived parameter rows (grain mix integer thresholds)
     bool grain_odd_state = false;           // grain mix: a state uploaded outside {+-0, +-0.5} (k_grain_mix until the next upload)
-    void *d_scratch = nullptr; size_t cap_scratch = 0;   // per-chunk start-state tables (XVOICE_SCAN)
+    void *d_scratch = nullptr; size_t cap_scratch = 0;   // per-chunk start-state tables (XVOICE_SCAN, GRAPH_SCAN); graph mix: group sums of a frame slice
     uint32_t *d_acc = nullptr; size_t cap_acc = 0;       // voice bank: integer accumulators of a bus split over tiles + tickets; all zero between launches
     unsigned long long *d_flags = nullptr;         // persistent-kernel progress words
     uint64_t n_flags = 0;

@@ -679,7 +679,117 @@ extern "C" __global__ void __launch_bounds__(128) graph_planar_simple(const Grap
     GRAPH_STORE_STATE(p.st, p.npad, i)
 }
 
-extern "C" __global__ void graph_planar_smem(uint32_t *out) { out[0] = WARPS * STAGES * STAGEB + WARPS * STAGES * 8; out[1] = WARPS * 32; out[2] = WARPS * STAGES * TT_STAGEB + WARPS * STAGES * 8 + 1024; }
+// Bus mix (io.mix; GraphMixParams as in k_graph.cu): one thread per instance for frames [m.t0, m.t0 + m.fc), MIX_CF frames
+// at a time, the per-instance outputs never leave registers.  The bus tree's first five levels run across the warp's lanes
+// as a recursive-halving transpose-reduce, lane bit 0 first (level 1 adds lanes 2m, 2m+1): at level b a lane keeps the half
+// of its frames that its lane bit b selects and adds the partner's sums for them -- one shuffle and one add per output per
+// instance-frame -- until every lane holds one frame, then butterflies for the lane bits left.  Lane r ends with frame
+// sum_b bit_b(r) * (MIX_CF >> (b + 1)).  The block's warps then add up in shared memory in groups of m.wg warps (the next
+// levels), and the group sums go to m.dst; k_graph_mix_tree does the levels above.  Lanes past n add the tree's padding,
+// -0.0f for a float and 0 for a w output, an exact identity.
+struct GraphMixParams { uint32_t *dst; uint64_t t0, fc, dst_F, dst_t0; uint32_t wg, outf; };   // must match k_graph.cu
+#define MIX_CF (GRAPH_NOUT <= 2 ? 16 : GRAPH_NOUT <= 4 ? 8 : 4)   // frames per transpose: MIX_CF * GRAPH_NOUT sums in registers
+#define MIX_WARPS 4
+#define MIX_F(q) ((GRAPH_OUTF >> (q)) & 1u)
+__device__ __forceinline__ uint32_t mix_add(uint32_t a, uint32_t b, bool f) {
+    return f ? __float_as_uint(__fadd_rn(__uint_as_float(a), __uint_as_float(b))) : a + b;
+}
+extern "C" __global__ void __launch_bounds__(MIX_WARPS * 32) graph_mix(const GraphParams p, const GraphMixParams m) {
+    __shared__ uint32_t red[2][MIX_WARPS][GRAPH_NOUT][MIX_CF];
+    const uint32_t lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    const bool mine = i < p.n;
+    GRAPH_DECL_STATE
+    GParam P = {};
+    if (mine) { GRAPH_LOAD_STATE(p.st, p.npad, i) GRAPH_LOAD_PARAM(p.prm, p.npad, i) }
+    const bool il = p.layout == 1;
+    const uint64_t n = p.n, t1 = m.t0 + m.fc;
+    uint32_t f_lane = 0;
+#pragma unroll
+    for (int b = 0, h = MIX_CF / 2; h >= 1; ++b, h >>= 1) f_lane += ((lane >> b) & 1u) * h;
+    // slices start at m.t0 + a multiple of MIX_CF, and m.t0 is 0 or a multiple of 32 (k_graph.cu)
+    const bool vec4 = ROWS_IN != 0 && !il && p.F % 4 == 0 && m.t0 % 4 == 0 && ((unsigned long long)p.in & 15) == 0 && ((unsigned long long)p.changed & 15) == 0;
+#pragma unroll 1
+    for (uint64_t tc = m.t0, c = 0; tc < t1; tc += MIX_CF, ++c) {
+        uint32_t v[GRAPH_NOUT][MIX_CF];
+        // the slice's input words are loaded before any tick, so their latencies overlap
+        uint32_t x[MIX_CF][GRAPH_NINA], g[MIX_CF];
+        if (vec4 && mine && tc + MIX_CF <= t1) {                         // PLANAR rows, 16-byte aligned: four frames per load
+#pragma unroll
+            for (int c = 0; c < MIX_CF / 4; ++c) {
+#pragma unroll
+                for (int j = 0; j < GRAPH_NIN; ++j) {
+                    const uint4 w = *(const uint4 *)(p.in + (i * GRAPH_NIN + j) * p.F + tc + 4 * c);
+                    x[4 * c][j] = w.x; x[4 * c + 1][j] = w.y; x[4 * c + 2][j] = w.z; x[4 * c + 3][j] = w.w;
+                }
+                uint4 w = make_uint4(0xFFFFFFFFu, 0xFFFFFFFFu, 0xFFFFFFFFu, 0xFFFFFFFFu);
+                if (GRAPH_HAS_CHANGED) w = *(const uint4 *)(p.changed + i * p.F + tc + 4 * c);
+                g[4 * c] = w.x; g[4 * c + 1] = w.y; g[4 * c + 2] = w.z; g[4 * c + 3] = w.w;
+            }
+        } else
+#pragma unroll
+        for (int k = 0; k < MIX_CF; ++k) {
+            const uint64_t t = tc + k;
+            const bool live = mine && t < t1;
+#pragma unroll
+            for (int j = 0; j < GRAPH_NIN; ++j) x[k][j] = !live ? 0u : il ? __ldcs(p.in + (t * GRAPH_NIN + j) * n + i) : p.in[(i * GRAPH_NIN + j) * p.F + t];
+            g[k] = GRAPH_HAS_CHANGED && live ? (il ? __ldcs(p.changed + t * n + i) : p.changed[i * p.F + t]) : 0xFFFFFFFFu;
+        }
+#pragma unroll
+        for (int k = 0; k < MIX_CF; ++k) {
+            const uint64_t t = tc + k;
+            uint32_t o[GRAPH_NOUT];
+            if (mine && t < t1) {
+                TICK(x[k], g[k], o);
+                if (p.out) {
+#pragma unroll
+                    for (int q = 0; q < GRAPH_NOUT; ++q) p.out[il ? (t * GRAPH_NOUT + q) * n + i : (i * GRAPH_NOUT + q) * p.F + t] = o[q];
+                }
+            } else {
+#pragma unroll
+                for (int q = 0; q < GRAPH_NOUT; ++q) o[q] = MIX_F(q) ? 0x80000000u : 0u;
+            }
+#pragma unroll
+            for (int q = 0; q < GRAPH_NOUT; ++q) v[q][k] = o[q];
+        }
+#pragma unroll
+        for (int b = 0, h = MIX_CF / 2; h >= 1; ++b, h >>= 1) {
+            const bool hi = (lane >> b) & 1u;
+#pragma unroll
+            for (int k = 0; k < h; ++k)
+#pragma unroll
+                for (int q = 0; q < GRAPH_NOUT; ++q) {
+                    const uint32_t send = hi ? v[q][k] : v[q][k + h], keep = hi ? v[q][k + h] : v[q][k];
+                    v[q][k] = mix_add(keep, __shfl_xor_sync(0xFFFFFFFFu, send, 1 << b), MIX_F(q));
+                }
+        }
+#pragma unroll
+        for (int b = 32 / MIX_CF; b > 1; b >>= 1)                       // lane bits above log2(MIX_CF)
+#pragma unroll
+            for (int q = 0; q < GRAPH_NOUT; ++q) v[q][0] = mix_add(v[q][0], __shfl_xor_sync(0xFFFFFFFFu, v[q][0], 32 / b), MIX_F(q));
+        if (lane < MIX_CF)
+#pragma unroll
+            for (int q = 0; q < GRAPH_NOUT; ++q) red[c & 1][warp][q][f_lane] = v[q][0];
+        __syncthreads();                                                 // red[c & 1] was last read in slice c - 2, before slice c - 1's barrier
+        const uint32_t per_block = MIX_WARPS >> (__ffs(m.wg) - 1);        // m.wg is a power of two
+        for (uint32_t e = threadIdx.x; e < per_block * GRAPH_NOUT * MIX_CF; e += blockDim.x) {
+            const uint32_t f = e % MIX_CF, q = (e / MIX_CF) % GRAPH_NOUT, gq = e / (MIX_CF * GRAPH_NOUT);
+            const bool isf = MIX_F(q);
+            uint32_t w[MIX_WARPS];
+#pragma unroll
+            for (int k = 0; k < MIX_WARPS; ++k) w[k] = k < (int)m.wg ? red[c & 1][gq * m.wg + k][q][f] : (isf ? 0x80000000u : 0u);
+#pragma unroll
+            for (int h = MIX_WARPS / 2; h >= 1; h >>= 1)
+#pragma unroll
+                for (int k = 0; k < h; ++k) w[k] = mix_add(w[2 * k], w[2 * k + 1], isf);
+            const uint64_t grp = (uint64_t)blockIdx.x * per_block + gq;
+            if (grp * 32 * m.wg < n && tc + f < t1) m.dst[(grp * GRAPH_NOUT + q) * m.dst_F + m.dst_t0 + (tc - m.t0) + f] = w[0];
+        }
+    }
+    if (mine) { GRAPH_STORE_STATE(p.st, p.npad, i) }
+}
+
+extern "C" __global__ void graph_planar_smem(uint32_t *out) { out[0] = WARPS * STAGES * STAGEB + WARPS * STAGES * 8; out[1] = WARPS * 32; out[2] = WARPS * STAGES * TT_STAGEB + WARPS * STAGES * 8 + 1024; out[3] = MIX_WARPS; }
 )SRC";
 
 }  // namespace
@@ -806,8 +916,10 @@ std::string cproc_graph_jit_source(const std::vector<cproc_cuda_node> &nodes, ui
     if (const char *e = getenv("CPROC_GRAPH_WARPS")) { const int v = atoi(e); if (v >= 1 && v <= 8) warps = v; }
     int hint = 0;
     if (const char *e = getenv("CPROC_GRAPH_ST_HINT")) hint = atoi(e) != 0;
-    snprintf(buf, sizeof(buf), "\n#define GRAPH_NOUT %zu\n#define GRAPH_NIN %u\n#define GRAPH_NINA %u\n#define GRAPH_HAS_CHANGED %d\n#define GRAPH_TF %d\n#define GRAPH_STAGES %d\n#define GRAPH_WARPS %d\n#define GRAPH_ST_HINT %d\n",
-             outs.size(), n_inputs, n_inputs ? n_inputs : 1u, has_changed ? 1 : 0, tf, stages, warps, hint);
+    uint32_t outf = 0;                                     // output q is a float: the node kind's out is (as in operand())
+    for (size_t q = 0; q < outs.size(); ++q) if (cproc_kind_out_float(nodes[outs[q]].type)) outf |= 1u << q;
+    snprintf(buf, sizeof(buf), "\n#define GRAPH_NOUT %zu\n#define GRAPH_NIN %u\n#define GRAPH_NINA %u\n#define GRAPH_HAS_CHANGED %d\n#define GRAPH_TF %d\n#define GRAPH_STAGES %d\n#define GRAPH_WARPS %d\n#define GRAPH_ST_HINT %d\n#define GRAPH_OUTF 0x%xu\n",
+             outs.size(), n_inputs, n_inputs ? n_inputs : 1u, has_changed ? 1 : 0, tf, stages, warps, hint, outf);
     // the tick text names the state words s<k>: they are members of the GState `S` in scope
     static const std::regex word("\\bs([0-9]+)\\b");
     tick = std::regex_replace(tick, word, "S.s$1");
@@ -849,14 +961,14 @@ int cproc_graph_jit_get(cproc_cuda_batch *b, bool has_changed, cproc_graph_jit *
         cudaKernel_t kq = nullptr;
         if (cudaLibraryGetKernel(&j.k_il, j.lib, "graph_interleaved") != cudaSuccess || cudaLibraryGetKernel(&j.k_pl, j.lib, "graph_planar") != cudaSuccess ||
             cudaLibraryGetKernel(&j.k_ps, j.lib, "graph_planar_simple") != cudaSuccess || cudaLibraryGetKernel(&j.k_pt, j.lib, "graph_planar_tma") != cudaSuccess ||
-            cudaLibraryGetKernel(&j.k_il4, j.lib, "graph_interleaved4") != cudaSuccess ||
+            cudaLibraryGetKernel(&j.k_il4, j.lib, "graph_interleaved4") != cudaSuccess || cudaLibraryGetKernel(&j.k_mix, j.lib, "graph_mix") != cudaSuccess ||
             cudaLibraryGetKernel(&kq, j.lib, "graph_planar_smem") != cudaSuccess) { cudaGetLastError(); b->jit_log = "cudaLibraryGetKernel failed"; return -1; }
-        // shared-memory size and block size of the planar kernel are defined by the generated source: ask it
-        uint32_t *d = nullptr, h[3] = {0, 0, 0};
-        if (cudaMalloc(&d, 12) != cudaSuccess) { cudaGetLastError(); return -1; }
+        // shared-memory size and block size of the planar kernels and the mix kernel's block are defined by the generated source: ask it
+        uint32_t *d = nullptr, h[4] = {0, 0, 0, 0};
+        if (cudaMalloc(&d, sizeof(h)) != cudaSuccess) { cudaGetLastError(); return -1; }
         void *args[] = {&d};
         cudaError_t e = cudaLaunchKernel((const void *)kq, dim3(1), dim3(1), args, 0, ctx->stream);
-        if (e == cudaSuccess) e = cudaMemcpyAsync(h, d, 12, cudaMemcpyDeviceToHost, ctx->stream);
+        if (e == cudaSuccess) e = cudaMemcpyAsync(h, d, sizeof(h), cudaMemcpyDeviceToHost, ctx->stream);
         if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
         cudaFree(d);
         if (e != cudaSuccess) { cudaGetLastError(); b->jit_log = "graph_planar_smem query failed"; return -1; }
@@ -864,6 +976,7 @@ int cproc_graph_jit_get(cproc_cuda_batch *b, bool has_changed, cproc_graph_jit *
         if (j.pl_smem > 227 * 1024) { b->jit_log = "planar staging does not fit shared memory (too many input streams)"; j.k_pl = nullptr; }
         else if (cudaFuncSetAttribute((const void *)j.k_pl, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)j.pl_smem) != cudaSuccess) { cudaGetLastError(); j.k_pl = nullptr; }
         j.pt_smem = h[2];
+        j.mix_warps = h[3];
         if (j.pt_smem > 227 * 1024 || cudaFuncSetAttribute((const void *)j.k_pt, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)j.pt_smem) != cudaSuccess) { cudaGetLastError(); j.k_pt = nullptr; }
         j.state = 1;
     }

@@ -28,6 +28,16 @@ struct GraphParams {
     const uint32_t *prm;           // SoA [param_words][npad]: the nodes' param structs in ANF order
 };
 
+// Bus mix of a GRAPH render (io.mix): the second argument of the mix kernels, here and in the generated source (graph_front.cu).
+// A mix kernel renders frames [t0, t0 + fc) and writes the sum of every tree group of 32 * wg instances (aligned to the bus
+// start) to dst[group][n_outputs][dst_F] at frame dst_t0 + (t - t0).
+struct GraphMixParams {
+    uint32_t *dst;
+    uint64_t t0, fc, dst_F, dst_t0;
+    uint32_t wg;                   // warps per tree group (power of two)
+    uint32_t outf;                 // bit q: output q is a float (summed with __fadd_rn), else a w (summed mod 2^32)
+};
+
 // acc_update (cproc.h:140-142) / edge_update (cproc.h:151-154) on register state
 // glide: mod_pdm_pwm.c:129-143 + mod_controlrate.c:28-40 on one parameter (see cproc_cuda.h)
 // extension processors: include/cproc_ext.h (x arrives already converted to the input's type: float inputs as float bits)
@@ -112,8 +122,14 @@ __global__ void k_graph_edge_acc(const GraphParams p, uint32_t mask) {
     for (int k = 0; k < DEPTH; ++k) p.st[(2 + k) * p.npad + i] = a[k];
 }
 
-// General table-driven graph.
-__global__ void k_graph_table(const GraphParams p) {
+__device__ __forceinline__ uint32_t mix_add(uint32_t a, uint32_t b, bool f) {
+    return f ? __float_as_uint(__fadd_rn(__uint_as_float(a), __uint_as_float(b))) : a + b;
+}
+
+// General table-driven graph.  MIX: frames [m.t0, m.t0 + m.fc) and every frame's sum over each warp's 32 instances (the first
+// five levels of the bus tree, lane bit 0 first: a butterfly gives every lane the same bits) to m.dst; out may be NULL.
+template <bool MIX>
+__global__ void k_graph_table(const GraphParams p, const GraphMixParams m) {
     __shared__ cproc_cuda_node nodes[GRAPH_MAX_NODES];
     __shared__ uint32_t off[GRAPH_MAX_NODES], poff[GRAPH_MAX_NODES], inf[GRAPH_MAX_NODES], outf[GRAPH_MAX_NODES], n_pw;
     if (threadIdx.x == 0) {
@@ -131,13 +147,18 @@ __global__ void k_graph_table(const GraphParams p) {
     }
     __syncthreads();
     const uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= p.n) return;
+    if (!MIX && i >= p.n) return;                                 // MIX: every lane takes part in the warp's shuffles
+    const bool mine = i < p.n;
     uint32_t s[GRAPH_MAX_STATE];
     uint32_t pr[GRAPH_MAX_PARAM];
-    for (uint32_t w = 0; w < p.state_words; ++w) s[w] = p.st[w * p.npad + i];
-    for (uint32_t w = 0; w < n_pw; ++w) pr[w] = p.prm[w * p.npad + i];
+    if (mine) {
+        for (uint32_t w = 0; w < p.state_words; ++w) s[w] = p.st[w * p.npad + i];
+        for (uint32_t w = 0; w < n_pw; ++w) pr[w] = p.prm[w * p.npad + i];
+    }
     const bool il = p.layout == CPROC_CUDA_INTERLEAVED;
-    for (uint64_t t = 0; t < p.F; ++t) {
+    const uint64_t t_end = MIX ? m.t0 + m.fc : p.F;
+    for (uint64_t t = MIX ? m.t0 : 0; t < t_end; ++t) {
+      if (mine) {
         const uint64_t oidx = il ? t * p.n + i : i * p.F + t;
         const uint32_t g = p.changed ? p.changed[oidx] : 0xFFFFFFFFu;
         for (uint32_t k = 0; k < p.n_nodes; ++k) {
@@ -154,16 +175,113 @@ __global__ void k_graph_table(const GraphParams p) {
             const uint32_t x2 = kd == CPROC_CUDA_NODE_PDM ? fetch(nodes[k].src2, false) : kd == CPROC_CUDA_NODE_MUL ? fetch(nodes[k].src2, true) : 0u;
             node_tick(nodes[k].type, s + off[k], pr + poff[k], x, x2);
         }
-        for (uint32_t q = 0; q < p.n_outputs; ++q)
-            p.out[il ? (t * p.n_outputs + q) * p.n + i : (i * p.n_outputs + q) * p.F + t] = s[off[p.out_nodes[q]]];
+        if (!MIX || p.out)
+            for (uint32_t q = 0; q < p.n_outputs; ++q)
+                p.out[il ? (t * p.n_outputs + q) * p.n + i : (i * p.n_outputs + q) * p.F + t] = s[off[p.out_nodes[q]]];
+      }
+        if (MIX) {
+            for (uint32_t q = 0; q < p.n_outputs; ++q) {
+                const bool f = (m.outf >> q) & 1u;
+                uint32_t v = mine ? s[off[p.out_nodes[q]]] : (f ? 0x80000000u : 0u);    // past n: the tree's -0.0f / 0 padding
+#pragma unroll
+                for (int b = 1; b < 32; b <<= 1) v = mix_add(v, __shfl_xor_sync(0xFFFFFFFFu, v, b), f);
+                if ((threadIdx.x & 31) == 0 && i < p.n)     // lane 0 of a warp with instances: warps past n have no group slot
+                    m.dst[((i >> 5) * p.n_outputs + q) * m.dst_F + m.dst_t0 + (t - m.t0)] = v;
+            }
+        }
     }
-    for (uint32_t w = 0; w < p.state_words; ++w) p.st[w * p.npad + i] = s[w];
+    if (mine)
+        for (uint32_t w = 0; w < p.state_words; ++w) p.st[w * p.npad + i] = s[w];
+}
+
+// One level range of the bus tree above the render kernels' groups: output slot j of bus b is the balanced tree over input
+// slots [32 j, 32 j + 32) of that bus, the slots past the bus's last padded with -0.0f / 0 (an exact identity).  src / dst:
+// [bus][slot][n_out][frames], src frame stride fc, dst frame stride dst_F at frame offset dst_t0.  The last bus has last_in
+// slots, the others gpb_in.  Serves the JIT mix kernels (the level above a block's groups) and the table kernel (above its warps).
+__global__ void k_graph_mix_tree(const uint32_t *src, uint32_t *dst, uint64_t n_bus, uint64_t gpb_in, uint64_t last_in, uint64_t gpb_out,
+                                 uint32_t n_out, uint64_t fc, uint64_t dst_F, uint64_t dst_t0, uint32_t outf) {
+    const uint64_t e = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (e >= n_bus * gpb_out * n_out * fc) return;
+    const uint64_t t = e % fc, q = (e / fc) % n_out, j = (e / (fc * n_out)) % gpb_out, b = e / (fc * n_out * gpb_out);
+    const uint64_t m = b == n_bus - 1 ? last_in : gpb_in, k0 = j * 32;
+    if (k0 >= m) return;
+    const bool f = (outf >> q) & 1u;
+    const uint32_t pad = f ? 0x80000000u : 0u;
+    uint32_t v[32];
+#pragma unroll
+    for (int w = 0; w < 32; ++w) v[w] = k0 + w < m ? src[((b * gpb_in + k0 + w) * n_out + q) * fc + t] : pad;
+#pragma unroll
+    for (int h = 16; h >= 1; h >>= 1)
+#pragma unroll
+        for (int w = 0; w < h; ++w) v[w] = mix_add(v[2 * w], v[2 * w + 1], f);
+    dst[((b * gpb_out + j) * n_out + q) * dst_F + dst_t0 + t] = v[0];
+}
+
+// io.mix: the render writes no per-instance stream unless io.out is set too; the tree groups of a render launch are summed
+// per bus by k_graph_mix_tree.  Frames go in slices whose partial sums stay under MIX_SCRATCH (mostly L2-resident between
+// the two launches); the tree depends on the bus's instance count only, so the slicing does not change a bit.
+#define MIX_SCRATCH (64ull << 20)
+static int launch_graph_mix(cproc_cuda_batch *b, uint64_t F, const cproc_cuda_io *io, GraphParams &p, cproc_graph_jit *j) {
+    cproc_cuda_ctx *ctx = b->ctx;
+    const uint64_t n = b->n, vpb = b->cfg.voices_per_bus;
+    const uint64_t span = vpb == 0 || vpb >= n ? n : vpb, n_bus = ceil_div_u64(n, span);
+    const uint32_t n_out = p.n_outputs;
+    uint32_t outf = 0;
+    for (uint32_t q = 0; q < n_out; ++q) if (cproc_kind_out_float(b->nodes[b->outs[q]].type)) outf |= 1u << q;
+    // tree group of a render launch: a warp (table kernel) or up to a whole block of the generated kernel, aligned to bus starts
+    const uint32_t warps = j ? j->mix_warps : 1;
+    uint32_t wg = warps;
+    while (wg > 1 && n_bus > 1 && span % (32ull * wg)) wg >>= 1;
+    const uint64_t g = 32ull * wg, gpb = ceil_div_u64(span, g), last_in = ceil_div_u64(n - (n_bus - 1) * span, g);
+    const uint64_t n_groups = (n_bus - 1) * gpb + last_in;
+    // scratch per frame: the render's group sums + the first tree level's output (the levels above reuse the first region)
+    const uint64_t per_frame = gpb == 1 ? 0 : 4ull * n_out * (n_groups + n_bus * ceil_div_u64(gpb, 32));
+    uint64_t fc = F;
+    if (per_frame && per_frame * F > MIX_SCRATCH) { fc = MIX_SCRATCH / per_frame / 32 * 32; if (fc < 32) fc = 32; if (fc > F) fc = F; }
+    if (per_frame * fc > b->cap_scratch) {
+        if (b->d_scratch) cudaFree(b->d_scratch);
+        b->d_scratch = nullptr; b->cap_scratch = 0;
+        // a period graph captured by cproc_cuda_run (abi.cu) holds the old scratch pointer: capture again
+        if (b->rg.exec) { cudaGraphExecDestroy(b->rg.exec); b->rg.exec = nullptr; b->rg.seen = 0; b->rg.F = 0; }
+        CK(ctx, cudaMalloc(&b->d_scratch, per_frame * fc));
+        b->cap_scratch = per_frame * fc;
+    }
+    uint32_t *bufA = (uint32_t *)b->d_scratch, *bufB = bufA + n_out * n_groups * fc;
+    for (uint64_t t0 = 0; t0 < F; t0 += fc) {
+        const uint64_t c = F - t0 < fc ? F - t0 : fc;
+        GraphMixParams m;
+        m.t0 = t0; m.fc = c; m.wg = wg; m.outf = outf;
+        if (gpb == 1) { m.dst = (uint32_t *)io->mix; m.dst_F = F; m.dst_t0 = t0; }
+        else { m.dst = bufA; m.dst_F = c; m.dst_t0 = 0; }
+        if (j) {
+            void *args[] = {&p, &m};
+            CK(ctx, cudaLaunchKernel((const void *)j->k_mix, dim3((unsigned)ceil_div_u64(n, 32ull * warps)), dim3(32 * warps), args, 0, ctx->stream));
+            ctx->launches++;
+        } else {
+            k_graph_table<true><<<(unsigned)ceil_div_u64(n, 128), 128, 0, ctx->stream>>>(p, m);
+            CK_LAUNCH(ctx, "k_graph_table (mix)");
+        }
+        uint32_t *src = bufA, *oth = bufB;
+        for (uint64_t gin = gpb, lin = last_in; gin > 1;) {
+            const uint64_t gout = ceil_div_u64(gin, 32), lout = ceil_div_u64(lin, 32);
+            const bool last = gout == 1;
+            uint32_t *dst = last ? (uint32_t *)io->mix : oth;
+            const uint64_t work = n_bus * gout * n_out * c;
+            k_graph_mix_tree<<<(unsigned)ceil_div_u64(work, 256), 256, 0, ctx->stream>>>(src, dst, n_bus, gin, lin, gout, n_out, c, last ? F : c, last ? t0 : 0, outf);
+            CK_LAUNCH(ctx, "k_graph_mix_tree");
+            oth = src; src = dst; gin = gout; lin = lout;
+        }
+    }
+    return 0;
 }
 
 int launch_graph(cproc_cuda_batch *b, uint64_t F, const cproc_cuda_io *io) {
     cproc_cuda_ctx *ctx = b->ctx;
-    if (!io->out || (!io->in && b->cfg.n_inputs)) return cproc_set_err(ctx, CPROC_CUDA_EINVAL, "graph: in/out is NULL");
+    if ((!io->out && !io->mix) || (!io->in && b->cfg.n_inputs)) return cproc_set_err(ctx, CPROC_CUDA_EINVAL, "graph: in/out is NULL");
     if (io->layout == CPROC_CUDA_TILED) return cproc_set_err(ctx, CPROC_CUDA_EINVAL, "graph: TILED layout not supported");
+    if (io->mix && b->cfg.voices_per_bus % 32)
+        return cproc_set_err(ctx, CPROC_CUDA_EINVAL, "graph mix: voices_per_bus %llu is neither 0 nor a multiple of 32", (unsigned long long)b->cfg.voices_per_bus);
+    if (io->mix && b->cfg.mode == CPROC_CUDA_GRAPH_SCAN) return cproc_set_err(ctx, CPROC_CUDA_EINVAL, "graph mix: not available in the GRAPH_SCAN mode");
     if (F == 0) return 0;
     if (b->cfg.mode == CPROC_CUDA_GRAPH_SCAN && F > 64) return launch_graph_scan(b, F, io);
     GraphParams p;
@@ -177,7 +295,11 @@ int launch_graph(cproc_cuda_batch *b, uint64_t F, const cproc_cuda_io *io) {
     const unsigned grid = (unsigned)ceil_div_u64(p.n, 128);
     // the kernel generated for this graph (graph_front.cu)
     cproc_graph_jit *j = nullptr;
-    if (ctx->graph_jit && cproc_graph_jit_get(b, p.changed != nullptr, &j) == 0) {
+    const bool jit = ctx->graph_jit && cproc_graph_jit_get(b, p.changed != nullptr, &j) == 0;
+    if (!jit && (b->nodes.size() > GRAPH_MAX_NODES || b->state_words > GRAPH_MAX_STATE || b->param_words > GRAPH_MAX_PARAM))
+        return cproc_set_err(ctx, CPROC_CUDA_EINVAL, "graph: %zu nodes need the NVRTC path, which is unavailable (%s)", b->nodes.size(), b->jit_log.c_str());
+    if (io->mix) return launch_graph_mix(b, F, io, p, jit ? j : nullptr);
+    if (jit) {
         void *args[] = {&p};
         cudaError_t e;
         CUtensorMap tin, tchg, tout;
@@ -194,8 +316,6 @@ int launch_graph(cproc_cuda_batch *b, uint64_t F, const cproc_cuda_io *io) {
         ctx->launches++;
         return cproc_check(ctx, e, "graph (jit)");
     }
-    if (b->nodes.size() > GRAPH_MAX_NODES || b->state_words > GRAPH_MAX_STATE || b->param_words > GRAPH_MAX_PARAM)
-        return cproc_set_err(ctx, CPROC_CUDA_EINVAL, "graph: %zu nodes need the NVRTC path, which is unavailable (%s)", b->nodes.size(), b->jit_log.c_str());
     // recognise edge -> acc [-> acc] chains under a single mask
     const std::vector<cproc_cuda_node> &nd = b->nodes;
     bool chain = nd.size() >= 2 && nd.size() <= 3 && nd[0].type == CPROC_CUDA_NODE_EDGE && nd[0].src == -1 &&
@@ -204,7 +324,7 @@ int launch_graph(cproc_cuda_batch *b, uint64_t F, const cproc_cuda_io *io) {
         chain = nd[k].type == CPROC_CUDA_NODE_ACC && nd[k].src == (int32_t)k - 1 && nd[k].cond_mask == nd[0].cond_mask;
     if (chain && nd.size() == 2) k_graph_edge_acc<1><<<grid, 128, 0, ctx->stream>>>(p, nd[0].cond_mask);
     else if (chain) k_graph_edge_acc<2><<<grid, 128, 0, ctx->stream>>>(p, nd[0].cond_mask);
-    else k_graph_table<<<grid, 128, 0, ctx->stream>>>(p);
+    else k_graph_table<false><<<grid, 128, 0, ctx->stream>>>(p, GraphMixParams{});
     CK_LAUNCH(ctx, "k_graph");
     return 0;
 }
