@@ -466,10 +466,10 @@ int  cproc_cuda_timer_start(cproc_cuda_ctx *ctx);
 int  cproc_cuda_timer_stop(cproc_cuda_ctx *ctx, float *elapsed_ms);
 /* Tuning knob by name; unknown names and out-of-range values return EINVAL.  Every setting gives
  * the same results (the tests sweep them); the defaults are the measured best on B200.
- *   planar_bulk      0..2 [2]  PLANAR square_grain / pdm / pwm / one-pole / word-clock / generated-graph streams:
+ *   planar_bulk      0/2  [2]  PLANAR square_grain / pdm / pwm / one-pole / word-clock / generated-graph streams:
  *                              0 = the register-transpose kernel for square_grain and the scalar kernels for the
- *                              others, 1 = per-lane cp.async.bulk staging, 2 = tensor-TMA staging; nonzero also
- *                              runs INTERLEAVED square_grain / pdm / one-pole four instances per thread
+ *                              others, 2 = tensor-TMA staging; 2 also runs INTERLEAVED square_grain / pdm / one-pole
+ *                              four instances per thread
  *   graph_vec4       0/1  [1]  INTERLEAVED generated graphs: four instances per thread (128-bit accesses)
  *   grain_mix2       0..2 [2]  square_grain mix kernel generation
  *   graph_jit        0/1  [1]  generated graphs compiled with NVRTC (0: table-driven kernel, <= 16 nodes)

@@ -108,7 +108,6 @@ int cproc_cuda_set_option(cproc_cuda_ctx *ctx, const char *name, int64_t value) 
     ctx->opt_epoch++;                                        // captured period graphs (cproc_cuda_run) are re-captured
     if (!strcmp(name, "pdm_block")) { if (value < 32 || value > 128 || (value & 31)) return cproc_set_err(ctx, CPROC_CUDA_EINVAL, "pdm_block must be 32, 64, 96 or 128"); ctx->pdm_block = (int)value; }
     else if (!strcmp(name, "pdm_tpb")) { if (value < 0 || value > 2) return cproc_set_err(ctx, CPROC_CUDA_EINVAL, "pdm_tpb must be 0 (thread per channel), 1 (thread per bank) or 2 (auto)"); ctx->pdm_tpb = (int)value; }
-    else if (!strcmp(name, "pdm_stage")) ctx->pdm_stage = value != 0;
     else if (!strcmp(name, "pdm_ws")) ctx->pdm_ws = value != 0;
     else if (!strcmp(name, "voice_fpt")) { if (value != 0 && value != 1 && value != 2 && value != 4 && value != 8 && value != 16) return cproc_set_err(ctx, CPROC_CUDA_EINVAL, "voice_fpt must be 0, 1, 2, 4, 8 or 16"); ctx->voice_fpt = (int)value; }
     else if (!strcmp(name, "pdm_tlog")) { if (value < 6 || value > 7) return cproc_set_err(ctx, CPROC_CUDA_EINVAL, "pdm_tlog must be 6 or 7"); ctx->pdm_tlog = (int)value; }
@@ -117,7 +116,7 @@ int cproc_cuda_set_option(cproc_cuda_ctx *ctx, const char *name, int64_t value) 
     else if (!strcmp(name, "pdm_ctas_per_sm")) { if (value < 1 || value > 8) return cproc_set_err(ctx, CPROC_CUDA_EINVAL, "pdm_ctas_per_sm must be 1..8"); ctx->pdm_ctas_per_sm = (int)value; }
     else if (!strcmp(name, "pdm_slice_batches")) { if (value < 2 || value > 65536) return cproc_set_err(ctx, CPROC_CUDA_EINVAL, "pdm_slice_batches must be 2..65536"); ctx->pdm_slice_batches = (int)value; }
     else if (!strcmp(name, "grain_blocks_per_sm")) { if (value < 1 || value > 16) return cproc_set_err(ctx, CPROC_CUDA_EINVAL, "grain_blocks_per_sm must be 1..16"); ctx->grain_blocks_per_sm = (int)value; }
-    else if (!strcmp(name, "planar_bulk")) { if (value < 0 || value > 2) return cproc_set_err(ctx, CPROC_CUDA_EINVAL, "planar_bulk must be 0..2"); ctx->planar_bulk = (int)value; }
+    else if (!strcmp(name, "planar_bulk")) { if (value != 0 && value != 2) return cproc_set_err(ctx, CPROC_CUDA_EINVAL, "planar_bulk must be 0 or 2"); ctx->planar_bulk = (int)value; }
     else if (!strcmp(name, "graph_vec4")) ctx->graph_vec4 = value != 0;
     else if (!strcmp(name, "graph_jit")) ctx->graph_jit = value != 0;
     else if (!strcmp(name, "grain_mix2")) { if (value < 0 || value > 2) return cproc_set_err(ctx, CPROC_CUDA_EINVAL, "grain_mix2 must be 0..2"); ctx->grain_mix2 = (int)value; }
@@ -445,7 +444,7 @@ int cproc_cuda_run(cproc_cuda_batch *b, uint64_t F, const cproc_cuda_io *io) {
     // accumulated with atomics: device memory only.
     // The graph mix kernel reads and writes per instance and frame: only a mix-only render without input streams qualifies
     // (its group sums go to the batch's device scratch, the bus mix straight to the staging).
-    const bool zc_ok = io->layout == CPROC_CUDA_PLANAR && ctx->planar_bulk >= 1 &&
+    const bool zc_ok = io->layout == CPROC_CUDA_PLANAR && ctx->planar_bulk != 0 &&
         (proc == CPROC_CUDA_VOICE_BANK ? io->mix == nullptr
          : proc == CPROC_CUDA_PWM ? F % 16 == 0
          : proc == CPROC_CUDA_GRAPH && io->mix ? !io->in && !io->in2 && !io->out

@@ -21,7 +21,6 @@ struct cproc_cuda_ctx {
     // tuning knobs (cproc_cuda_set_option)
     int pdm_block = 64;       // threads per block of the PDM kernels
     int pdm_tpb = 2;          // plain PDM kernels, banks of <= 4: 1 thread per bank, 0 thread per channel (every thread replays its bank's generator), 2 auto
-    int pdm_stage = 1;        // 1: smem-staged full-line stores for PLANAR
     int pdm_ws = 1;           // PDM v2: 1 = producer / consumer kernel under the dynamic (group, slice) schedule (k_pdm_v2_ws4), 0 = plain thread-per-bank / per-channel kernels
     int pdm_tlog = 7;         // k_pdm_v2_ws4: log2 of the dither batch (ticks per FULL / EMPTY hand-off), 6 or 7
     int pdm_v1_chains = 2;    // v1 thread-per-bank TILED kernels: PRNG chains per lane (1 or 2)
@@ -36,10 +35,9 @@ struct cproc_cuda_ctx {
     int pdm_warps_per_smsp = 1;
     int n_sm = CPROC_N_SM;
     int voice_fpt = 0;        // voice bank: frames per thread (0 = by frame count; 1, 2, 4, 8)
-    int grain_block = 128;
     int grain_blocks_per_sm = 2;
     int grain_mix2 = 2;       // 0: float kernel; 1: register-accumulator / integer-threshold kernel; 2: predicate-state kernel
-    int planar_bulk = 2;      // square_grain / pdm_raw / onepole / pwm streams through planar_bulk.cuh: 0 off, 1 per-lane bulk copies, 2 tensor TMA (PLANAR); nonzero: k_interleaved4 (INTERLEAVED)
+    int planar_bulk = 2;      // square_grain / pdm_raw / onepole / pwm / word-clock / generated-graph streams: 0 scalar kernels, 2 tensor-TMA staging (PLANAR), k_interleaved4 (INTERLEAVED)
     int graph_vec4 = 1;       // interleaved generated graphs: four instances per thread when n % 4 == 0
     int graph_jit = 1;        // 1: generated graphs are compiled with NVRTC; 0: table-driven kernel
     int xvoice_vpt = 0;       // k_xvoice_mix: voices per thread per L2-resident tile (0 = default)
@@ -58,8 +56,8 @@ struct cproc_graph_jit {
     int state = 0;
     std::vector<char> cubin;
     cudaLibrary_t lib = nullptr;
-    cudaKernel_t k_il = nullptr, k_il4 = nullptr, k_pl = nullptr, k_ps = nullptr, k_pt = nullptr, k_mix = nullptr;
-    uint32_t pl_smem = 0, pl_block = 0, pt_smem = 0, mix_warps = 0;   // mix_warps: block of the bus-mix kernel graph_mix, in warps
+    cudaKernel_t k_il = nullptr, k_il4 = nullptr, k_ps = nullptr, k_pt = nullptr, k_mix = nullptr;
+    uint32_t pt_block = 0, pt_smem = 0, mix_warps = 0;   // block and shared memory of graph_planar_tma; mix_warps: block of the bus-mix kernel graph_mix, in warps
 };
 
 struct cproc_cuda_bus;

@@ -15,7 +15,7 @@
 //    generates CUDA source for exactly this graph (every node state word a named
 //    register, every source a literal register name, masks as immediates) and compiles
 //    it with NVRTC for sm_100a when the batch is created.  PLANAR streams are staged
-//    with per-lane bulk copies as in pbulk::k_planar_bulk; INTERLEAVED streams are read in
+//    with tensor TMA as in pbulk::k_planar_tma; INTERLEAVED streams are read in
 //    16-frame batches.  libnvrtc is loaded with dlopen: without it (or with graph_jit=0)
 //    graphs of up to 16 nodes run on the table-driven kernel of k_graph.cu.
 #include "common.cuh"
@@ -468,94 +468,18 @@ extern "C" __global__ void __launch_bounds__(128) graph_interleaved4(const Graph
     GRAPH_STORE_STATE4(p.st, p.npad, i)
 }
 
-// [inst][n_inputs][F] in, [inst][F] changed / out (what a host hands over): lane r of a warp
-// owns instance r of the warp's 32 and stages ITS rows through shared memory with bulk
-// copies (cp.async.bulk + mbarrier), one row segment of TF frames per stream per tile;
-// the output overwrites the row of input 0 in place and leaves with one bulk store.
 __device__ __forceinline__ uint32_t smem_u32(const void *q) { return (uint32_t)__cvta_generic_to_shared(q); }
 #define TF GRAPH_TF                 // frames per tile: 64, or 32 for graphs with many instructions per tick (more resident warps)
 #define ROWS_IN (GRAPH_NIN + (GRAPH_HAS_CHANGED ? 1 : 0))
 #define ROWS (ROWS_IN > GRAPH_NOUT ? ROWS_IN : GRAPH_NOUT)   // output q overwrites row q in place
-#define ROWB (TF * 4 + 16)
-#define STAGEB (32 * ROWS * ROWB)
 #define STAGES GRAPH_STAGES
 #define WARPS GRAPH_WARPS
-extern "C" __global__ void __launch_bounds__(WARPS * 32) graph_planar(const GraphParams p) {
-    extern __shared__ __align__(128) unsigned char sm[];
-    const uint32_t lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    const uint64_t g0 = ((uint64_t)blockIdx.x * WARPS + warp) * 32;
-    if (g0 >= p.n) return;
-    const uint32_t rows = p.n - g0 < 32 ? (uint32_t)(p.n - g0) : 32u;
-    const bool mine = lane < rows;
-    const uint64_t i = g0 + lane;
-    const uint32_t base = smem_u32(sm) + warp * (STAGES * STAGEB);
-    const uint32_t bar0 = smem_u32(sm) + WARPS * STAGES * STAGEB + warp * (STAGES * 8);
-    if (lane == 0) {
-#pragma unroll
-        for (int s = 0; s < STAGES; ++s) asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(bar0 + 8 * s), "r"(1));
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
-    __syncwarp();
-    GRAPH_DECL_STATE
-    GParam P = {};
-    if (mine) { GRAPH_LOAD_STATE(p.st, p.npad, i) GRAPH_LOAD_PARAM(p.prm, p.npad, i) }
-    const uint32_t n_tiles = (uint32_t)((p.F + TF - 1) / TF);
-    auto cols_of = [&](uint32_t k) { const uint64_t left = p.F - (uint64_t)k * TF; return left < TF ? (uint32_t)left : (uint32_t)TF; };
-    auto issue = [&](uint32_t k) {
-        const uint32_t s = k % STAGES, bytes = cols_of(k) * 4;
-        if (lane == 0) asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar0 + 8 * s), "r"(rows * ROWS_IN * bytes) : "memory");
-        if (mine) {
-#pragma unroll
-            for (int j = 0; j < ROWS_IN; ++j) {
-                const uint32_t *srow = j < GRAPH_NIN ? p.in + (i * GRAPH_NIN + j) * p.F : p.changed + i * p.F;
-                asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-                             ::"r"(base + s * STAGEB + (j * 32 + lane) * ROWB), "l"(srow + (uint64_t)k * TF), "r"(bytes), "r"(bar0 + 8 * s) : "memory");
-            }
-        }
-    };
-#pragma unroll 1
-    for (uint32_t k = 0; k + 2 < STAGES && k < n_tiles; ++k) issue(k);
-#pragma unroll 1
-    for (uint32_t k = 0; k < n_tiles; ++k) {
-        if (k + STAGES - 2 < n_tiles) {                   // that stage last held tile k-2: its bulk store must have read it out
-            asm volatile("cp.async.bulk.wait_group.read 1;" ::: "memory");
-            __syncwarp();
-            issue(k + STAGES - 2);
-        }
-        const uint32_t s = k % STAGES, cols = cols_of(k);
-        asm volatile("{\n\t.reg .pred q;\n\tW: mbarrier.try_wait.parity.shared::cta.b64 q, [%0], %1;\n\t@q bra D;\n\tbra W;\n\tD:\n\t}"
-                     ::"r"(bar0 + 8 * s), "r"((k / STAGES) & 1) : "memory");
-        const uint32_t row = base + s * STAGEB + lane * ROWB;      // stream j of this lane: row + j * 32 * ROWB
-        if (mine) {
-            for (uint32_t c = 0; c < cols / 4; ++c) {
-                // four frames per 128-bit access; separate arrays and explicit ticks keep every index static
-                uint32_t xa[GRAPH_NINA], xb[GRAPH_NINA], xc[GRAPH_NINA], xd[GRAPH_NINA], ga = 0xFFFFFFFFu, gb = 0xFFFFFFFFu, gc = 0xFFFFFFFFu, gd = 0xFFFFFFFFu;
-                uint32_t oa[GRAPH_NOUT], ob[GRAPH_NOUT], oc[GRAPH_NOUT], od[GRAPH_NOUT];
-#pragma unroll
-                for (int j = 0; j < GRAPH_NIN; ++j)
-                    asm volatile("ld.shared.v4.u32 {%0, %1, %2, %3}, [%4];" : "=r"(xa[j]), "=r"(xb[j]), "=r"(xc[j]), "=r"(xd[j]) : "r"(row + j * (32 * ROWB) + 16 * c));
-                if (GRAPH_HAS_CHANGED)
-                    asm volatile("ld.shared.v4.u32 {%0, %1, %2, %3}, [%4];" : "=r"(ga), "=r"(gb), "=r"(gc), "=r"(gd) : "r"(row + GRAPH_NIN * (32 * ROWB) + 16 * c));
-                TICK(xa, ga, oa); TICK(xb, gb, ob); TICK(xc, gc, oc); TICK(xd, gd, od);
-#pragma unroll
-                for (int q = 0; q < GRAPH_NOUT; ++q)
-                    asm volatile("st.shared.v4.u32 [%0], {%1, %2, %3, %4};" ::"r"(row + q * (32 * ROWB) + 16 * c), "r"(oa[q]), "r"(ob[q]), "r"(oc[q]), "r"(od[q]) : "memory");
-            }
-            asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-#pragma unroll
-            for (int q = 0; q < GRAPH_NOUT; ++q)
-                asm volatile("cp.async.bulk.global.shared::cta.bulk_group [%0], [%1], %2;" ::"l"(p.out + (i * GRAPH_NOUT + q) * p.F + (uint64_t)k * TF), "r"(row + q * (32 * ROWB)), "r"(cols * 4) : "memory");
-        }
-        asm volatile("cp.async.bulk.commit_group;" ::: "memory");
-    }
-    asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");
-    if (mine) { GRAPH_STORE_STATE(p.st, p.npad, i) }
-}
 
-// The same staging with TENSOR TMA (planar_bulk.cuh, k_planar_tma): the streams are 3-D tensors
-// [inst][stream][F], a box is 32 frames x 1 stream x 32 instances (SWIZZLE_128B), ONE elected lane moves
-// the two boxes of every stream of a 64-frame tile (the per-lane bulk copies above are executed one lane
-// at a time by the uniform datapath), lane r finds 16-byte chunk c of its row at r*128 + ((c ^ (r&7)) << 4).
+// [inst][n_inputs][F] in, [inst][F] changed / out (what a host hands over), staged through shared memory with TENSOR TMA
+// (planar_bulk.cuh, k_planar_tma): lane r of a warp owns instance r of the warp's 32.  The streams are 3-D tensors
+// [inst][stream][F], a box is 32 frames x 1 stream x 32 instances (SWIZZLE_128B), ONE elected lane moves the TF / 32 boxes
+// of every stream of a tile, lane r finds 16-byte chunk c of its row at r*128 + ((c ^ (r&7)) << 4); output q
+// overwrites the row of stream q in place and leaves with tensor-TMA stores.
 struct __align__(64) CUtensorMap { unsigned long long opaque[16]; };
 #define TT_BOXB 4096
 #define TT_STREAMB ((TF / 32) * TT_BOXB)
@@ -789,7 +713,7 @@ extern "C" __global__ void __launch_bounds__(MIX_WARPS * 32) graph_mix(const Gra
     if (mine) { GRAPH_STORE_STATE(p.st, p.npad, i) }
 }
 
-extern "C" __global__ void graph_planar_smem(uint32_t *out) { out[0] = WARPS * STAGES * STAGEB + WARPS * STAGES * 8; out[1] = WARPS * 32; out[2] = WARPS * STAGES * TT_STAGEB + WARPS * STAGES * 8 + 1024; out[3] = MIX_WARPS; }
+extern "C" __global__ void graph_planar_smem(uint32_t *out) { out[0] = WARPS * 32; out[1] = WARPS * STAGES * TT_STAGEB + WARPS * STAGES * 8 + 1024; out[2] = MIX_WARPS; }
 )SRC";
 
 }  // namespace
@@ -959,12 +883,12 @@ int cproc_graph_jit_get(cproc_cuda_batch *b, bool has_changed, cproc_graph_jit *
         }
         if (cudaLibraryLoadData(&j.lib, j.cubin.data(), nullptr, nullptr, 0, nullptr, nullptr, 0) != cudaSuccess) { cudaGetLastError(); b->jit_log = "cudaLibraryLoadData failed"; return -1; }
         cudaKernel_t kq = nullptr;
-        if (cudaLibraryGetKernel(&j.k_il, j.lib, "graph_interleaved") != cudaSuccess || cudaLibraryGetKernel(&j.k_pl, j.lib, "graph_planar") != cudaSuccess ||
+        if (cudaLibraryGetKernel(&j.k_il, j.lib, "graph_interleaved") != cudaSuccess ||
             cudaLibraryGetKernel(&j.k_ps, j.lib, "graph_planar_simple") != cudaSuccess || cudaLibraryGetKernel(&j.k_pt, j.lib, "graph_planar_tma") != cudaSuccess ||
             cudaLibraryGetKernel(&j.k_il4, j.lib, "graph_interleaved4") != cudaSuccess || cudaLibraryGetKernel(&j.k_mix, j.lib, "graph_mix") != cudaSuccess ||
             cudaLibraryGetKernel(&kq, j.lib, "graph_planar_smem") != cudaSuccess) { cudaGetLastError(); b->jit_log = "cudaLibraryGetKernel failed"; return -1; }
-        // shared-memory size and block size of the planar kernels and the mix kernel's block are defined by the generated source: ask it
-        uint32_t *d = nullptr, h[4] = {0, 0, 0, 0};
+        // block and shared-memory size of graph_planar_tma and the mix kernel's block are defined by the generated source: ask it
+        uint32_t *d = nullptr, h[3] = {0, 0, 0};
         if (cudaMalloc(&d, sizeof(h)) != cudaSuccess) { cudaGetLastError(); return -1; }
         void *args[] = {&d};
         cudaError_t e = cudaLaunchKernel((const void *)kq, dim3(1), dim3(1), args, 0, ctx->stream);
@@ -972,12 +896,9 @@ int cproc_graph_jit_get(cproc_cuda_batch *b, bool has_changed, cproc_graph_jit *
         if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
         cudaFree(d);
         if (e != cudaSuccess) { cudaGetLastError(); b->jit_log = "graph_planar_smem query failed"; return -1; }
-        j.pl_smem = h[0]; j.pl_block = h[1];
-        if (j.pl_smem > 227 * 1024) { b->jit_log = "planar staging does not fit shared memory (too many input streams)"; j.k_pl = nullptr; }
-        else if (cudaFuncSetAttribute((const void *)j.k_pl, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)j.pl_smem) != cudaSuccess) { cudaGetLastError(); j.k_pl = nullptr; }
-        j.pt_smem = h[2];
-        j.mix_warps = h[3];
-        if (j.pt_smem > 227 * 1024 || cudaFuncSetAttribute((const void *)j.k_pt, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)j.pt_smem) != cudaSuccess) { cudaGetLastError(); j.k_pt = nullptr; }
+        j.pt_block = h[0]; j.pt_smem = h[1]; j.mix_warps = h[2];
+        if (j.pt_smem > 227 * 1024) { b->jit_log = "planar staging does not fit shared memory (too many input streams)"; j.k_pt = nullptr; }
+        else if (cudaFuncSetAttribute((const void *)j.k_pt, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)j.pt_smem) != cudaSuccess) { cudaGetLastError(); j.k_pt = nullptr; }
         j.state = 1;
     }
     *out = &j;

@@ -35,9 +35,7 @@ int launch_word_clock(cproc_cuda_batch *b, uint64_t F, const cproc_cuda_io *io) 
     if (io->layout == CPROC_CUDA_TILED) return cproc_set_err(ctx, CPROC_CUDA_EINVAL, "word_clock: TILED layout not supported");
     if (F == 0) return 0;
     WordClockOp op; op.st = b->d_state; op.prm = b->d_param; op.npad = b->npad; op.phase = 0; op.pol = 0; op.h = 0;
-    if (ctx->planar_bulk && io->layout == CPROC_CUDA_PLANAR && pbulk::usable(F, io->out, io->out)) {
-        int rc = pbulk::launch<64, 3>(ctx, op, (const uint32_t *)io->out, (uint32_t *)io->out, b->n, F);
-        if (rc) return rc;
+    if (ctx->planar_bulk && io->layout == CPROC_CUDA_PLANAR && pbulk::launch(ctx, op, (const uint32_t *)io->out, (uint32_t *)io->out, b->n, F)) {
         CK_LAUNCH(ctx, "k_word_clock (planar template)");
         return 0;
     }

@@ -10,7 +10,7 @@
 // the grain axis carries the parallelism (one thread per grain).
 //
 // GrainOp: PLANAR [grain][F] streams go through the staging templates of
-//   planar_bulk.cuh (k_planar_tma, k_planar_bulk), INTERLEAVED [F][grain] streams
+//   planar_bulk.cuh (k_planar_tma), INTERLEAVED [F][grain] streams
 //   through k_interleaved4 (four grains per thread), as the other stream processors.
 // k_grain_planar: the PLANAR fallback (planar_bulk = 0, F % 4 != 0 or rows off
 //   16-byte alignment).  A warp owns 32 grains and walks the frame axis in 32-frame
@@ -112,9 +112,7 @@ int launch_square_grain(cproc_cuda_batch *b, uint64_t F, const cproc_cuda_io *io
     if (io->layout == CPROC_CUDA_TILED) return cproc_set_err(ctx, CPROC_CUDA_EINVAL, "square_grain: TILED layout not supported");
     if (F == 0) return 0;
     GrainOp op; op.state = (float *)b->d_state; op.thresh = (const float *)b->d_param; op.st = 0.f; op.th = 0.f;
-    if (ctx->planar_bulk && io->layout == CPROC_CUDA_PLANAR && pbulk::usable(F, io->in, io->out)) {
-        int rc = pbulk::launch<64, 3>(ctx, op, (const uint32_t *)io->in, (uint32_t *)io->out, b->n, F);
-        if (rc) return rc;
+    if (ctx->planar_bulk && io->layout == CPROC_CUDA_PLANAR && pbulk::launch(ctx, op, (const uint32_t *)io->in, (uint32_t *)io->out, b->n, F)) {
         CK_LAUNCH(ctx, "k_grain (bulk)");
         return 0;
     }

@@ -307,12 +307,11 @@ int launch_graph(cproc_cuda_batch *b, uint64_t F, const cproc_cuda_io *io) {
         const bool vec4 = ctx->graph_vec4 && p.n % 4 == 0 && ((uintptr_t)p.in & 15) == 0 && ((uintptr_t)p.out & 15) == 0 && (!p.changed || ((uintptr_t)p.changed & 15) == 0);
         if (io->layout == CPROC_CUDA_INTERLEAVED && vec4) e = cudaLaunchKernel((const void *)j->k_il4, dim3((unsigned)ceil_div_u64(p.n, 512)), dim3(128), args, 0, ctx->stream);
         else if (io->layout == CPROC_CUDA_INTERLEAVED) e = cudaLaunchKernel((const void *)j->k_il, dim3(grid), dim3(128), args, 0, ctx->stream);
-        else if (j->k_pt && aligned && ctx->planar_bulk >= 2 && pbulk::encode_rows3_u32(&tin, p.n_inputs ? p.in : p.out, F, p.n_inputs ? p.n_inputs : p.n_outputs, p.n) &&
+        else if (j->k_pt && aligned && ctx->planar_bulk && pbulk::encode_rows3_u32(&tin, p.n_inputs ? p.in : p.out, F, p.n_inputs ? p.n_inputs : p.n_outputs, p.n) &&
                  pbulk::encode_rows3_u32(&tchg, p.changed ? p.changed : (p.n_inputs ? p.in : p.out), F, 1, p.n) && pbulk::encode_rows3_u32(&tout, p.out, F, p.n_outputs, p.n)) {
             void *targs[] = {&p, &tin, &tchg, &tout};
-            e = cudaLaunchKernel((const void *)j->k_pt, dim3((unsigned)ceil_div_u64(p.n, j->pl_block)), dim3(j->pl_block), targs, j->pt_smem, ctx->stream);
-        } else if (j->k_pl && aligned) e = cudaLaunchKernel((const void *)j->k_pl, dim3((unsigned)ceil_div_u64(p.n, j->pl_block)), dim3(j->pl_block), args, j->pl_smem, ctx->stream);
-        else e = cudaLaunchKernel((const void *)j->k_ps, dim3(grid), dim3(128), args, 0, ctx->stream);
+            e = cudaLaunchKernel((const void *)j->k_pt, dim3((unsigned)ceil_div_u64(p.n, j->pt_block)), dim3(j->pt_block), targs, j->pt_smem, ctx->stream);
+        } else e = cudaLaunchKernel((const void *)j->k_ps, dim3(grid), dim3(128), args, 0, ctx->stream);
         ctx->launches++;
         return cproc_check(ctx, e, "graph (jit)");
     }

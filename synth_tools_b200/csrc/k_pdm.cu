@@ -127,41 +127,13 @@ __device__ __forceinline__ void v1_word(const uint32_t (&sp)[B], uint32_t (&acc)
     for (int j = 0; j < B; ++j) wv[j] = __brev(bits[j]);
 }
 
-// The same word with the bank's generator run as TWO interleaved chains: xorshift32 is a 6-deep
+// The same word with the bank's generator run as TWO interleaved chains (xorshift32 is a 6-deep
 // dependent chain per tick and there are fewer than two warps per scheduler at the C2 shape, so
-// one chain leaves the issue slots idle.  Chain A produces ticks 0..15, chain B -- started 16
-// steps ahead with the GF(2) jump table M^16 -- ticks 16..31 into registers; the accumulators
-// then consume them in time order.
-template <int B>
-__device__ __forceinline__ void v1_word2(const uint32_t (&sp)[B], uint32_t (&acc)[B], uint32_t &rng, const uint32_t (*jt)[256],
-                                         uint32_t dmask, uint32_t (&wv)[B]) {
-    uint32_t bits[B], late[16];
-#pragma unroll
-    for (int j = 0; j < B; ++j) bits[j] = 0;
-    uint32_t xa = rng, xb = jump_apply(jt, rng);
-#pragma unroll
-    for (int i = 0; i < 16; ++i) {
-        xa = xorshift32_step(xa);
-        xb = xorshift32_step(xb);
-        late[i] = xb & dmask;
-        const uint32_t d = xa & dmask;                                             // mod_pdm.c:261
-#pragma unroll
-        for (int j = 0; j < B; ++j) add_carry_shift(acc[j], bits[j], sp[j] + d);   // :235-240
-    }
-#pragma unroll
-    for (int i = 0; i < 16; ++i) {
-#pragma unroll
-        for (int j = 0; j < B; ++j) add_carry_shift(acc[j], bits[j], sp[j] + late[i]);
-    }
-    rng = xb;
-#pragma unroll
-    for (int j = 0; j < B; ++j) wv[j] = __brev(bits[j]);
-}
-
-// Software-pipelined form of the two-chain word: while the accumulators consume the 32 dither
-// values of word w (registers `cur`), the generator produces the 32 values of word w+1 (`nxt`) --
-// chain A ticks 0..15, chain B (started with the jump table M^16) ticks 16..31.  The accumulate
-// chain (one dependent add per tick) is then never paced by the 6-deep xorshift chain.
+// one chain leaves the issue slots idle), software pipelined: while the accumulators consume the
+// 32 dither values of word w (registers `cur`), the generator produces the 32 values of word w+1
+// (`nxt`) -- chain A ticks 0..15, chain B (started 16 steps ahead with the GF(2) jump table M^16)
+// ticks 16..31.  The accumulate chain (one dependent add per tick) is then never paced by the
+// 6-deep xorshift chain.
 // GEN = false for the last word of a group: nothing is generated beyond it.
 template <int B, bool GEN>
 __device__ __forceinline__ void v1_word_pipe(const uint32_t (&sp)[B], uint32_t (&acc)[B], const uint32_t (&cur)[32], uint32_t (&nxt)[32],
@@ -411,7 +383,7 @@ __global__ void k_pdm_raw(const PdmRawParams p) {
     for (int k = 0; k < K; ++k) p.st[k * p.npad + c] = s[k];
 }
 
-// PLANAR streams through the bulk-staged template (planar_bulk.cuh): the per-thread row walk of
+// PLANAR streams through the staging template (planar_bulk.cuh): the per-thread row walk of
 // k_pdm_raw touches 32 different lines per warp instruction.
 template <int K, int HAS_IN>
 struct PdmRawOp {
@@ -434,13 +406,13 @@ struct PdmRawOp {
 };
 
 template <int K>
-static int launch_pdm_raw_bulk(cproc_cuda_ctx *ctx, const PdmRawParams &p) {
+static bool launch_pdm_raw_bulk(cproc_cuda_ctx *ctx, const PdmRawParams &p) {
     if (p.in) {
         PdmRawOp<K, 1> op; op.st = p.st; op.param = p.param; op.dither = p.dither; op.npad = p.npad; op.sh = p.sh;
-        return pbulk::launch<64, 3>(ctx, op, p.in, p.out, p.n, p.F);
+        return pbulk::launch(ctx, op, p.in, p.out, p.n, p.F);
     }
     PdmRawOp<K, 0> op; op.st = p.st; op.param = p.param; op.dither = p.dither; op.npad = p.npad; op.sh = p.sh;
-    return pbulk::launch<64, 3>(ctx, op, p.out, p.out, p.n, p.F);
+    return pbulk::launch(ctx, op, p.out, p.out, p.n, p.F);
 }
 
 template <int K>
@@ -464,17 +436,18 @@ int launch_pdm(cproc_cuda_batch *b, uint64_t F, const cproc_cuda_io *io) {
     p.in = (const uint32_t *)io->in; p.dither = (const uint32_t *)io->in2; p.out = (uint32_t *)io->out;
     p.F = F; p.sh = b->cfg.out_shift; p.layout = io->layout;
     unsigned grid = (unsigned)ceil_div_u64(p.n, 128);
-    if (ctx->planar_bulk && io->layout == CPROC_CUDA_PLANAR && pbulk::usable(F, p.in, p.out)) {
-        int rc;
+    if (ctx->planar_bulk && io->layout == CPROC_CUDA_PLANAR) {
+        bool staged;
         switch (b->cfg.order) {
-        case 1: rc = launch_pdm_raw_bulk<1>(ctx, p); break;
-        case 2: rc = launch_pdm_raw_bulk<2>(ctx, p); break;
-        case 3: rc = launch_pdm_raw_bulk<3>(ctx, p); break;
-        default: rc = launch_pdm_raw_bulk<4>(ctx, p); break;
+        case 1: staged = launch_pdm_raw_bulk<1>(ctx, p); break;
+        case 2: staged = launch_pdm_raw_bulk<2>(ctx, p); break;
+        case 3: staged = launch_pdm_raw_bulk<3>(ctx, p); break;
+        default: staged = launch_pdm_raw_bulk<4>(ctx, p); break;
         }
-        if (rc) return rc;
-        CK_LAUNCH(ctx, "k_pdm_raw (bulk)");
-        return 0;
+        if (staged) {
+            CK_LAUNCH(ctx, "k_pdm_raw (bulk)");
+            return 0;
+        }
     }
     if (ctx->planar_bulk && io->layout == CPROC_CUDA_INTERLEAVED && pbulk::usable_interleaved4(p.n, p.in, p.out)) {
         switch (b->cfg.order) {
@@ -511,7 +484,7 @@ __global__ void k_pwm(uint32_t *phase, const uint32_t *speed, uint64_t n, uint64
     phase[c] = ph;
 }
 
-// PLANAR duty bytes through the bulk-staged template: one "frame" of the template is a 32-bit word
+// PLANAR duty bytes through the staging template: one "frame" of the template is a 32-bit word
 // = four ticks (duty is 8 bit), so a lane's 64-word tile is 256 ticks of its channel.
 struct PwmOp {
     static constexpr int NIN = 0;
@@ -562,10 +535,8 @@ int launch_pwm(cproc_cuda_batch *b, uint64_t F, const cproc_cuda_io *io) {
         CK_LAUNCH(ctx, "k_pwm_tiled");
         return 0;
     }
-    if (ctx->planar_bulk && io->layout == CPROC_CUDA_PLANAR && F % 16 == 0 && pbulk::usable(F / 4, io->out, io->out)) {
-        PwmOp op; op.phase = b->d_state; op.speed = b->d_param; op.ph = 0; op.sp = 0;
-        int rc = pbulk::launch<64, 3>(ctx, op, (const uint32_t *)io->out, (uint32_t *)io->out, b->n, F / 4);
-        if (rc) return rc;
+    PwmOp op; op.phase = b->d_state; op.speed = b->d_param; op.ph = 0; op.sp = 0;
+    if (ctx->planar_bulk && io->layout == CPROC_CUDA_PLANAR && F % 16 == 0 && pbulk::launch(ctx, op, (const uint32_t *)io->out, (uint32_t *)io->out, b->n, F / 4)) {
         CK_LAUNCH(ctx, "k_pwm (bulk)");
         return 0;
     }

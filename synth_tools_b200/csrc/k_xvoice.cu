@@ -1362,15 +1362,12 @@ int launch_onepole(cproc_cuda_batch *b, uint64_t F, const cproc_cuda_io *io) {
         if (L < 64 && ctx->xvoice_chunk <= 0) L = 64;
         if (L < F) return launch_onepole_scan(b, F, io, L);
     }
-    if (ctx->planar_bulk && io->layout == CPROC_CUDA_PLANAR && pbulk::usable(F, io->in, io->out)) {
-        OnepoleOp op; op.y = (float *)b->d_state; op.a = (const float *)b->d_param; op.s = 0.f; op.c = 0.f;
-        int rc = pbulk::launch<64, 3>(ctx, op, (const uint32_t *)io->in, (uint32_t *)io->out, b->n, F);
-        if (rc) return rc;
+    OnepoleOp op; op.y = (float *)b->d_state; op.a = (const float *)b->d_param; op.s = 0.f; op.c = 0.f;
+    if (ctx->planar_bulk && io->layout == CPROC_CUDA_PLANAR && pbulk::launch(ctx, op, (const uint32_t *)io->in, (uint32_t *)io->out, b->n, F)) {
         CK_LAUNCH(ctx, "k_onepole (bulk)");
         return 0;
     }
     if (ctx->planar_bulk && io->layout == CPROC_CUDA_INTERLEAVED && pbulk::usable_interleaved4(b->n, io->in, io->out)) {
-        OnepoleOp op; op.y = (float *)b->d_state; op.a = (const float *)b->d_param; op.s = 0.f; op.c = 0.f;
         pbulk::launch_interleaved4(ctx, op, (const uint32_t *)io->in, (uint32_t *)io->out, b->n, F);
         CK_LAUNCH(ctx, "k_onepole (interleaved4)");
         return 0;

@@ -1,17 +1,19 @@
-// planar_bulk.cuh -- generic bulk-staged render of PLANAR 32-bit streams ([inst][F], what
-// the reference hosts hand over), shared by square_grain, pdm raw, pwm, the one-pole and the
-// word clock.  Lane r of a warp owns instance r of the warp's 32; per tile of TF frames the lane issues
-// one bulk copy (cp.async.bulk, the non-tensor TMA path) of ITS row segment into its row
-// of a shared-memory stage, walks the row with LDS.128 / STS.128 in place, and sends it
-// back with one bulk store.  Loads run one tile ahead, stores drain one tile behind.
+// planar_bulk.cuh -- generic staged render of PLANAR 32-bit streams ([inst][F], what the
+// reference hosts hand over), shared by square_grain, pdm raw, pwm, the one-pole and the word
+// clock.  Lane r of a warp owns instance r of the warp's 32.  The stream is a 2-D tensor
+// [inst][F] (box = 32 words x 32 instances, SWIZZLE_128B): per tile of 64 frames one elected
+// lane moves the warp's two boxes into a shared-memory stage with two tensor-TMA copies, every
+// lane walks its row with LDS.128 / STS.128 in place -- lane r finds 16-byte chunk c of its row
+// at r*128 + ((c ^ (r & 7)) << 4) -- and the elected lane sends the tile back with two tensor-TMA
+// stores.  Loads run one tile ahead, stores drain one tile behind.
 //
 // Op (by value, trivially copyable):
 //   static constexpr int NIN      0: no per-instance input stream (output only), 1: one
 //   void     load(uint64_t i)     state / params of instance i from the SoA rows
 //   void     store(uint64_t i)
 //   uint32_t tick(uint32_t x, uint64_t t)   one frame; x = the input word (NIN == 1)
-// Requirements (checked by the launcher): F % 4 == 0, in/out 16-byte aligned; in may alias
-// out exactly.
+// Requirements (checked by launch, which declines otherwise): F % 4 == 0, in/out 16-byte
+// aligned; in may alias out exactly.
 #pragma once
 #include "common.cuh"
 #include <cuda.h>
@@ -26,80 +28,7 @@ __device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity) {
 }
 
 constexpr int WARPS = 2;
-template <int TF, int STAGES> constexpr size_t smem_bytes() { return (size_t)WARPS * STAGES * 32 * (TF * 4 + 16) + WARPS * STAGES * 8; }
 
-template <int TF, int STAGES, class Op>
-__global__ void __launch_bounds__(WARPS * 32) k_planar_bulk(Op op, const uint32_t *in, uint32_t *out, uint64_t n, uint64_t F) {
-    constexpr uint32_t ROWB = TF * 4 + 16;              // 16-byte units of 8 consecutive lanes fall in 8 different bank groups
-    constexpr uint32_t STAGEB = 32 * ROWB;
-    extern __shared__ __align__(128) uint8_t pb_smem[];
-    const uint32_t lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    const uint64_t g0 = ((uint64_t)blockIdx.x * WARPS + warp) * 32;
-    if (g0 >= n) return;
-    const uint32_t rows = n - g0 < 32 ? (uint32_t)(n - g0) : 32u;
-    const bool mine = lane < rows;
-    const uint64_t i = g0 + lane;
-    const uint32_t base = smem_u32(pb_smem) + warp * (STAGES * STAGEB);
-    const uint32_t bar0 = smem_u32(pb_smem) + WARPS * STAGES * STAGEB + warp * (STAGES * 8);
-    if (Op::NIN && lane == 0) {
-#pragma unroll
-        for (int s = 0; s < STAGES; ++s) asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(bar0 + 8 * s), "r"(1));
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
-    __syncwarp();
-    if (mine) op.load(i);
-    const uint32_t *src = in + i * F;
-    uint32_t *dst = out + i * F;
-    const uint32_t n_tiles = (uint32_t)((F + TF - 1) / TF);
-    auto cols_of = [&](uint32_t k) { const uint64_t left = F - (uint64_t)k * TF; return left < TF ? (uint32_t)left : (uint32_t)TF; };
-    auto issue = [&](uint32_t k) {
-        const uint32_t s = k % STAGES, bytes = cols_of(k) * 4;
-        if (lane == 0) asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar0 + 8 * s), "r"(rows * bytes) : "memory");
-        if (mine) asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-                               ::"r"(base + s * STAGEB + lane * ROWB), "l"(src + (uint64_t)k * TF), "r"(bytes), "r"(bar0 + 8 * s) : "memory");
-    };
-    if (Op::NIN) {
-#pragma unroll 1
-        for (uint32_t k = 0; k < STAGES - 2 && k < n_tiles; ++k) issue(k);
-    }
-#pragma unroll 1
-    for (uint32_t k = 0; k < n_tiles; ++k) {
-        const uint32_t s = k % STAGES, cols = cols_of(k);
-        if (Op::NIN) {
-            if (k + STAGES - 2 < n_tiles) {               // that stage last held tile k-2: its bulk store must have read it out
-                asm volatile("cp.async.bulk.wait_group.read 1;" ::: "memory");
-                __syncwarp();
-                issue(k + STAGES - 2);
-            }
-            mbar_wait(bar0 + 8 * s, (k / STAGES) & 1);
-        } else {
-            asm volatile("cp.async.bulk.wait_group.read %0;" ::"n"(STAGES - 1) : "memory");   // the store of tile k-STAGES has left this stage
-        }
-        const uint32_t row = base + s * STAGEB + lane * ROWB;
-        if (mine) {
-            const uint64_t t0 = (uint64_t)k * TF;
-#pragma unroll 4
-            for (uint32_t c = 0; c < cols / 4; ++c) {
-                uint32_t x0 = 0, x1 = 0, x2 = 0, x3 = 0;
-                if (Op::NIN) asm volatile("ld.shared.v4.u32 {%0, %1, %2, %3}, [%4];" : "=r"(x0), "=r"(x1), "=r"(x2), "=r"(x3) : "r"(row + 16 * c));
-                const uint64_t t = t0 + 4 * c;
-                x0 = op.tick(x0, t); x1 = op.tick(x1, t + 1); x2 = op.tick(x2, t + 2); x3 = op.tick(x3, t + 3);
-                asm volatile("st.shared.v4.u32 [%0], {%1, %2, %3, %4};" ::"r"(row + 16 * c), "r"(x0), "r"(x1), "r"(x2), "r"(x3) : "memory");
-            }
-            asm volatile("fence.proxy.async.shared::cta;" ::: "memory");     // generic-proxy row writes -> visible to the bulk store
-            asm volatile("cp.async.bulk.global.shared::cta.bulk_group [%0], [%1], %2;" ::"l"(dst + t0), "r"(row), "r"(cols * 4) : "memory");
-        }
-        asm volatile("cp.async.bulk.commit_group;" ::: "memory");
-    }
-    asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");
-    if (mine) op.store(i);
-}
-
-// ---- tensor-TMA form --------------------------------------------------------------------------
-// Per-lane bulk copies are executed one lane at a time by the uniform datapath (most of the warp
-// instructions of k_planar_bulk are copy issue).  With a 2-D tensor map over the [inst][F] stream
-// (box = 32 words x 32 instances, SWIZZLE_128B) one elected lane moves a whole 32 x 64 tile with
-// two instructions, and lane r finds 16-byte chunk c of its row at r*128 + ((c ^ (r & 7)) << 4).
 typedef CUresult (*encode_tiled_t)(CUtensorMap *, CUtensorMapDataType, cuuint32_t, void *, const cuuint64_t *, const cuuint64_t *, const cuuint32_t *,
                                    const cuuint32_t *, CUtensorMapInterleave, CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
 inline encode_tiled_t encode_fn() {
@@ -217,30 +146,20 @@ __global__ void __launch_bounds__(WARPS * 32) k_planar_tma(Op op, const __grid_c
     if (mine) op.store(g0 + lane);
 }
 
-inline bool usable(uint64_t F, const void *in, const void *out) {
-    return F % 4 == 0 && ((uintptr_t)in & 15) == 0 && ((uintptr_t)out & 15) == 0;
-}
-
-template <int TF, int STAGES, class Op>
-int launch(cproc_cuda_ctx *ctx, const Op &op, const uint32_t *in, uint32_t *out, uint64_t n, uint64_t F) {
+// Renders the streams with k_planar_tma and returns true, or returns false when they cannot be staged (F % 4 != 0, a
+// stream off 16-byte alignment, or no tensor map encodes them): the caller then runs its scalar kernel.  A CUDA error is
+// left for the caller's launch check (CK_LAUNCH).
+template <class Op>
+bool launch(cproc_cuda_ctx *ctx, const Op &op, const uint32_t *in, uint32_t *out, uint64_t n, uint64_t F) {
     CUtensorMap tin, tout;
-    if (ctx->planar_bulk >= 2 && encode_rows_u32(&tout, out, F, n) && encode_rows_u32(&tin, Op::NIN ? (const void *)in : (const void *)out, F, n)) {
-        static bool tset[64] = {};
-        if (!tset[ctx->device & 63]) {
-            CK(ctx, cudaFuncSetAttribute(k_planar_tma<Op>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)t_smem_bytes()));
-            tset[ctx->device & 63] = true;
-        }
-        k_planar_tma<Op><<<(unsigned)ceil_div_u64(n, WARPS * 32), WARPS * 32, t_smem_bytes(), ctx->stream>>>(op, tin, tout, n, F);
-        return 0;
-    }
-    constexpr size_t smem = smem_bytes<TF, STAGES>();
+    if (!encode_rows_u32(&tout, out, F, n) || !encode_rows_u32(&tin, Op::NIN ? (const void *)in : (const void *)out, F, n)) return false;
     static bool attr_set[64] = {};
     if (!attr_set[ctx->device & 63]) {
-        CK(ctx, cudaFuncSetAttribute(k_planar_bulk<TF, STAGES, Op>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        if (cudaFuncSetAttribute(k_planar_tma<Op>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)t_smem_bytes()) != cudaSuccess) return true;
         attr_set[ctx->device & 63] = true;
     }
-    k_planar_bulk<TF, STAGES, Op><<<(unsigned)ceil_div_u64(n, WARPS * 32), WARPS * 32, smem, ctx->stream>>>(op, in, out, n, F);
-    return 0;
+    k_planar_tma<Op><<<(unsigned)ceil_div_u64(n, WARPS * 32), WARPS * 32, t_smem_bytes(), ctx->stream>>>(op, tin, tout, n, F);
+    return true;
 }
 
 // ---- INTERLEAVED streams [F][inst]: four adjacent instances per thread ---------------------------------------------------

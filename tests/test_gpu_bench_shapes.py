@@ -393,7 +393,7 @@ def test_c2_v1_bench_shape(gpu, oracle):
 
 def test_pdm_raw_bench_shape(gpu, oracle):
     """pdm_raw: pdm2_update (order 2, shift 24) on 1 Mi channels x 1,024 ticks, 4 GiB in and 4 GiB out.  PLANAR through
-    tensor-TMA staging (planar_bulk 2) and through per-lane bulk copies (planar_bulk 1) write identical streams, and the
+    tensor-TMA staging (planar_bulk 2) and through the scalar k_pdm_raw (planar_bulk 0) write identical streams, and the
     INTERLEAVED render (k_interleaved4) is their transpose.  The input repeats bench's 16,384-row chunk; the channels
     differ through their integrator states, so the oracle on the sampled channels sees every channel's own output."""
     torch, st, ctx = gpu.torch, gpu.st, gpu.ctx
@@ -405,7 +405,7 @@ def test_pdm_raw_bench_shape(gpu, oracle):
     try:
         bufs["in"] = gpu.put(chunk).repeat(N // 16384, 1)                      # [ch][F]
         bufs["in_il"] = bufs["in"].t().contiguous()                             # [F][ch]
-        for name, layout, mode in (("planar_tma", "PLANAR", 2), ("planar_bulk", "PLANAR", 1), ("interleaved", "INTERLEAVED", 2)):
+        for name, layout, mode in (("planar_tma", "PLANAR", 2), ("planar_scalar", "PLANAR", 0), ("interleaved", "INTERLEAVED", 2)):
             b = ctx.batch(st.PDM, N, order=order, out_shift=24, layout=getattr(st, layout))
             try:
                 b.upload_state(s0)
@@ -416,7 +416,7 @@ def test_pdm_raw_bench_shape(gpu, oracle):
                 ends[name] = b.download_state()
             finally:
                 b.free()
-        assert same(torch, bufs["planar_tma"], bufs["planar_bulk"])
+        assert same(torch, bufs["planar_tma"], bufs["planar_scalar"])
         assert torch.equal(bufs["interleaved"].view(F, N).t(), bufs["planar_tma"].view(N, F))
         for name, s in ends.items():
             assert np.array_equal(s, ends["planar_tma"]), name
@@ -448,7 +448,7 @@ BP5_TEXT = """#define CPROC_NB_INPUTS 1
 
 def test_graph_bp5_bench_shape(gpu, oracle):
     """graph_bp5: the generated edge -> acc -> acc graph, 4 Mi instances x 256 ticks, 4 GiB per stream.  The NVRTC kernels
-    (PLANAR with tensor-TMA and with per-lane bulk staging, INTERLEAVED) and the library's own chain kernel (graph_jit 0)
+    (PLANAR with tensor-TMA staging and the scalar graph_planar_simple, INTERLEAVED) and the library's own chain kernel (graph_jit 0)
     agree on the device; the oracle reproduces instances around 2^20 and 2^21 and the last ones up to 2^22 - 1 (PLANAR rows
     above 3 GiB from 2^22 - 2^20 on; INTERLEAVED ticks >= 128 above 2 GiB).  Every instance starts from its own state."""
     torch, st, ctx = gpu.torch, gpu.st, gpu.ctx
@@ -463,7 +463,7 @@ def test_graph_bp5_bench_shape(gpu, oracle):
     try:
         bufs["in"] = gpu.put(chunk).repeat(N // 65536, 1)                      # [inst][1][F]
         bufs["in_il"] = bufs["in"].t().contiguous()                             # [F][1][inst]
-        for name, layout, opts in (("jit_tma", "PLANAR", {"planar_bulk": 2}), ("jit_bulk", "PLANAR", {"planar_bulk": 1}),
+        for name, layout, opts in (("jit_tma", "PLANAR", {"planar_bulk": 2}), ("jit_simple", "PLANAR", {"planar_bulk": 0}),
                                    ("jit_il", "INTERLEAVED", {}), ("chain_kernel", "PLANAR", {"graph_jit": 0})):
             with options(ctx, **opts):
                 b = ctx.batch(st.GRAPH, N, nodes=rows, n_inputs=n_in, out_node=out_node, layout=getattr(st, layout))
@@ -476,7 +476,7 @@ def test_graph_bp5_bench_shape(gpu, oracle):
                     ends[name] = b.download_state()
                 finally:
                     b.free()
-        for name in ("jit_bulk", "chain_kernel"):
+        for name in ("jit_simple", "chain_kernel"):
             assert same(torch, bufs["jit_tma"], bufs[name]), name
         assert torch.equal(bufs["jit_il"].view(F, N).t(), bufs["jit_tma"].view(N, F))
         for name, s in ends.items():

@@ -372,9 +372,9 @@ def _n_sm():
 @pytest.mark.gpu
 @pytest.mark.parametrize("inplace", [False, True], ids=["out-of-place", "in-place"])
 @pytest.mark.parametrize("layout,N,F", [("PLANAR", 300, 256), ("PLANAR", 300, 203), ("INTERLEAVED", 256, 100), ("INTERLEAVED", 301, 77)])
-@pytest.mark.parametrize("bulk", [0, 1, 2])
+@pytest.mark.parametrize("bulk", [0, 2])
 def test_square_grain_edges(st, ctx, oracle, bulk, layout, N, F, inplace):
-    """Raw square_grain on every stream path (planar_bulk 0..2; F and N multiples of 4 or not), two blocks.  The outputs
+    """Raw square_grain on every stream path (planar_bulk 0 or 2; F and N multiples of 4 or not), two blocks.  The outputs
     are copies of the state, so the comparison is bitwise, NaN payloads included."""
     s0, th, _ = _grain_edge_inputs(N, F)
     il = layout == "INTERLEAVED"
@@ -575,7 +575,7 @@ def onepole_edge_inputs(N, F):
 
 @pytest.mark.gpu
 @pytest.mark.parametrize("layout,N,F", [("PLANAR", 52, 256), ("PLANAR", 53, 203), ("INTERLEAVED", 52, 160), ("INTERLEAVED", 53, 77)])
-@pytest.mark.parametrize("bulk", [0, 1, 2])
+@pytest.mark.parametrize("bulk", [0, 2])
 def test_onepole_edges(st, ctx, oracle, bulk, layout, N, F):
     """Sequential one-pole on every stream path: coefficients 0, -0, subnormal, 2^-24, 0.5, 1, 2, 3 (unstable: to inf,
     then NaN), inf, NaN; pool inputs, overflowing inputs, subnormal inputs and a decay through the subnormal range to
@@ -754,7 +754,7 @@ def test_xvoice_mix2_lp_zero_sign(st, ctx, oracle):
 
 # ------------------------------------------------------------------------------------------------ GPU: extension graphs
 # kernel -> (layout, N, F, planar_bulk, graph_jit): how the front end is steered to it (k_graph.cu launch_graph)
-GRAPH_KERNELS = {"graph_planar_tma": (0, 300, 256, 2, 1), "graph_planar": (0, 300, 256, 1, 1),
+GRAPH_KERNELS = {"graph_planar_tma": (0, 300, 256, 2, 1),
                  "graph_planar_simple": (0, 131, 203, 2, 1), "graph_interleaved4": (1, 256, 100, 2, 1),
                  "graph_interleaved": (1, 301, 77, 2, 1), "table": (0, 131, 96, 2, 0)}
 

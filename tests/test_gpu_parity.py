@@ -375,11 +375,14 @@ def test_pwm_layouts(st, ctx, oracle, N, F, layout):
     b.free()
 
 
-@pytest.mark.parametrize("mode", [0, 1, 2])
+@pytest.mark.parametrize("mode", [0, 2])
 @pytest.mark.parametrize("N,F", [(130, 320), (33, 64), (1000, 1024), (70, 100), (5, 36)])
 def test_planar_template_modes(st, ctx, oracle, mode, N, F):
-    """pdm raw (with and without an input stream), one-pole and pwm through the scalar kernels (0), the
-    per-lane bulk-copy template (1) and its tensor-TMA form (2): ragged instance counts and tiles."""
+    """pdm raw (with and without an input stream), one-pole and pwm through the scalar kernels (0) and the
+    tensor-TMA staging template (2): ragged instance counts and tiles."""
+    for name, value in (("planar_bulk", 1), ("pdm_stage", 1)):      # planar_bulk takes 0 or 2; pdm_stage is no option
+        with pytest.raises(st.CprocCudaError):
+            ctx.set_option(name, value)
     ctx.set_option("planar_bulk", mode)
     try:
         for order in (1, 3):
@@ -892,13 +895,13 @@ def test_square_grain_interleaved_variants(st, ctx, oracle, mode, N, F):
         ctx.set_option("planar_bulk", 2)
 
 
-@pytest.mark.parametrize("mode", [0, 1, 2])
+@pytest.mark.parametrize("mode", [0, 2])
 @pytest.mark.parametrize("N,F,neg_th,odd", [(1000, 256, False, False), (77, 100, False, False), (300, 1024, True, False),
                                             (64, 4, False, True), (4097, 64, True, True), (31, 392, False, False)])
 def test_square_grain_bulk_variants(st, ctx, oracle, mode, N, F, neg_th, odd):
-    """The PLANAR kernels by planar_bulk (0 register transpose, 1 per-lane bulk copies, 2 tensor
-    TMA): ragged last tiles, ragged last warp, negative thresholds and non-reference state values
-    (both take the literal two-branch form)."""
+    """The PLANAR kernels by planar_bulk (0 register transpose, 2 tensor TMA): ragged last tiles,
+    ragged last warp, negative thresholds and non-reference state values (both take the literal
+    two-branch form)."""
     ctx.set_option("planar_bulk", mode)
     try:
         _square_grain_case(st, ctx, oracle, N, F, "PLANAR", neg_th, odd)
@@ -1063,11 +1066,11 @@ def test_xvoice_scan_zero_state_forms(st, ctx, oracle, closed, layout, groups):
         ctx.set_option("xvoice_chunk", 0); ctx.set_option("xvoice_groups", 0); ctx.set_option("xvoice_closed", 1)
 
 
-@pytest.mark.parametrize("N,F,chunk,groups,mode", [(70, 1001, 32, 0, 2), (200, 3000, 96, 0, 1), (700, 2048, 32, 3, 1), (40, 2050, 64, 0, 2), (500, 998, 32, 4, 2)])
+@pytest.mark.parametrize("N,F,chunk,groups,mode", [(70, 1001, 32, 0, 2), (200, 3000, 96, 0, 2), (700, 2048, 32, 3, 2), (40, 2050, 64, 0, 2), (500, 998, 32, 4, 2)])
 def test_xvoice_scan_planar_store_paths(st, ctx, oracle, N, F, chunk, groups, mode):
-    """PLANAR render: tensor-TMA stores (planar_bulk 2, even F) and the staged-row kernel it falls back to
-    (odd F, planar_bulk 1) agree with the sequential oracle to 1e-5 of the peak at benign filters (the
-    per-voice contract against the fp64 filter: tests/test_gpu_float_ref.py)."""
+    """PLANAR render: tensor-TMA stores (even F) and the staged-row kernel it falls back to (odd F) agree
+    with the sequential oracle to 1e-5 of the peak at benign filters (the per-voice contract against the
+    fp64 filter: tests/test_gpu_float_ref.py)."""
     s0, prm = _xvoice_inputs(oracle, N)
     prm["gate_frames"] = rng.integers(0, F, N)
     sa = s0.copy()

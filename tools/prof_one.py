@@ -146,7 +146,7 @@ elif which == "pdmraw":
     chunk = rng.integers(0, 2**32, (16384, F), dtype=np.uint32)
     for k in range(N // 16384):
         ctx.h2d(d_in + k * chunk.nbytes, chunk)
-    for mode in (0, 1, 2):
+    for mode in (0, 2):
         ctx.set_option("planar_bulk", mode)
         b = ctx.batch(st.PDM, N, order=2, out_shift=24)
         ms = timed(lambda: b.run_dev(F, inp=d_in, out=d_out))

@@ -6,4 +6,3 @@ for tf in 32 64; do for st in 2 3 4 5; do for w in 1 2 3 4; do
   CPROC_GRAPH_TF=$tf CPROC_GRAPH_STAGES=$st CPROC_GRAPH_WARPS=$w timeout 120 python tools/prof_one.py gvoice 3 2>&1 | tail -1
 done; done; done
 echo -n "default  "; timeout 120 python tools/prof_one.py gvoice 3 2>&1 | tail -1
-for tf in 32 64; do echo -n "per-lane bulk copies (planar_bulk=1) TF=$tf  "; CPROC_GRAPH_TF=$tf timeout 120 python tools/prof_one.py gvoice 3 planar_bulk=1 2>&1 | tail -1; done
